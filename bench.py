@@ -2,7 +2,7 @@
 """bench.py -- pose queries/sec (encode + codebook NN) on 128x128 crops (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision simt|tc]
-                    [--workload infer|sharded|routed|train|process] [--batches-per-step M]
+                    [--workload infer|sharded|routed|train|process] [--batches-per-step M] [--dump-outputs DIR]
 
 infer (default, BASELINE.json configs[1]): one BATCH = 256 synthetic uint8 crops through the hot path: conv encoder -> latent
     -> fused L2-normalise + cosine match against the 92 232-row codebook -> (score, index) per crop.  One "step" = M (default
@@ -27,6 +27,9 @@ Printed JSON (rank 0, one line):
   parity     one-off check outside the timed region: 10 000 crops, tensor-core path vs the exact-order fp32 path
   cpu_baseline     the CPU oracle (restated reference path, variables resident, best thread count) on this box's cores
 --impl reference times that CPU path as the whole arm (TensorFlow is not installable offline: oracle port).
+--dump-outputs DIR (infer): after the timed steps rank 0 writes what its last timed step returned, stacked over the step's M
+    batches: DIR/scores.npy (float32 [M, 256, 1]) and DIR/indices.npy (codebook rows as float64 [M, 256, 1]).  Weights,
+    codebook and crops are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -462,6 +465,13 @@ def parity_check(sess, cb, dev, n_queries=10000):
             "against": "this library's AAE_PREC_FP32_SIMT path (exact fp32 operation order; itself index-exact vs the CPU oracle in tests/)"}
 
 
+def dump_outputs(out_dir, batches):
+    """Writes the (scores, idx) pairs Codebook.nearest_idx_device returned for `batches`, stacked in batch order."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "scores.npy"), np.stack([s.cpu().numpy() for s, _ in batches]))
+    np.save(os.path.join(out_dir, "indices.npy"), np.stack([i.cpu().numpy() for _, i in batches]).astype(np.float64))
+
+
 def run_ours(args, rank, world, local_rank):
     import ctypes as C
 
@@ -527,17 +537,24 @@ def run_ours(args, rank, world, local_rank):
     torch.cuda.synchronize()
     launches0 = lib.aae_launch_count()
     evs = []
+    dump = args.dump_outputs is not None and rank == 0
+    last_step = []
     for i in range(n_batches):
         flush.zero_()
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record()
-        batch_device(i)
+        res = batch_device(i)
         b.record()
         evs.append((a, b))
+        if dump and i >= n_batches - M:
+            last_step.append(res)
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
     launches = lib.aae_launch_count() - launches0
+    if dump:
+        dump_outputs(args.dump_outputs, last_step)
+        del last_step
     batch_ms = [a.elapsed_time(b) for a, b in evs]
     total_ms = max_over_ranks(sum(batch_ms), dev, world)
 
@@ -900,7 +917,15 @@ def main():
     ap.add_argument("--no-collective-workloads", action="store_true")
     ap.add_argument("--batches-per-step", type=int, default=16)
     ap.add_argument("--workload", default="infer", choices=["infer", "train", "sharded", "routed", "process"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR/*.npy (infer workload)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None:
+        if args.impl != "ours" or args.workload != "infer":
+            ap.error("--dump-outputs is implemented for --impl ours --workload infer only")
+        if max(1, args.batches_per_step) * BATCH * (4 + 8) > 64 * 10**6:    # float32 scores + float64 indices of one step
+            ap.error("--dump-outputs writes whole steps: at most %d batches per step" % (64 * 10**6 // (BATCH * 12)))
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -9,6 +9,8 @@ HEADER_PATH = os.path.join(_HERE, "..", "include", "aae_b200.h")
 AAE_MAX_LAYERS = 8
 PREC_FP32_SIMT = 0
 PREC_TC_SPLIT = 1
+RENDER_VIEW_FLOATS = 64
+RENDER_BEHIND_CAMERA, RENDER_EMPTY, RENDER_BAD_CROP = 1, 2, 4
 
 
 class AaeError(RuntimeError):
@@ -69,6 +71,11 @@ _SIGS = {
     "aae_trainer_set_global_step": (_I, [_P, _L]),
     "aae_extract_square_patches": (_I, [_P, _I, _I, _P, _I, _F, _I, _P, _P]),
     "aae_augment_batch": (_I, [_P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P]),
+    "aae_mesh_create": (_I, [_I, _P, _L, _P, _L, C.POINTER(_P)]),
+    "aae_mesh_destroy": (_I, [_P]),
+    "aae_render_workspace_bytes": (_L, [_P, _I, _I, _I]),
+    "aae_render_frames": (_I, [_P, _P, _I, _I, _I, _F, _F, _P, _L, _P, _P, _P, _P, _P]),
+    "aae_render_crops": (_I, [_P, _P, _I, _I, _I, _F, _F, _P, C.c_double, _I, _I, _P, _P, _P, _L, _P, _P, _P, _P, _P, _P]),
 }
 
 _lib = None

@@ -123,9 +123,10 @@ def gaussian_taps_q8(sigma):
     return kq
 
 
-def nearest_cells(dst, src):
+def nearest_cells(dst, src, dtype=np.uint8):
+    """cv2.resize INTER_NEAREST: source index of each of the dst output cells for a source of src cells"""
     ifx = 1.0 / (float(dst) / float(src))
-    return np.minimum(np.floor(np.arange(dst, dtype=np.float64) * ifx).astype(np.int64), src - 1).astype(np.uint8)
+    return np.minimum(np.floor(np.arange(dst, dtype=np.float64) * ifx).astype(np.int64), src - 1).astype(dtype)
 
 
 _IDENT = np.arange(256, dtype=np.uint8)

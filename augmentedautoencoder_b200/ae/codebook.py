@@ -205,7 +205,10 @@ class Codebook(object):
         return sess.run(fetch, {self._encoder.x: x}).squeeze()
 
     def update_embedding(self, session, batch_size):
-        """Build the codebook: encode every rendered view, L2-normalise in float64, store fp32 (codebook.py:190-219)."""
+        """Build the codebook: encode every rendered view, L2-normalise in float64, store fp32 (codebook.py:190-219).  With the
+        dataset's CUDA renderer the uint8 crops go from the renderer to the encoder without a host round trip."""
+        if getattr(self._dataset, "has_gpu_renderer", False):
+            return self._update_embedding(session, batch_size, self._dataset.embedding_crops_device)
         return self._update_embedding(session, batch_size, self._dataset.render_embedding_image_batch)
 
     def update_embedding_from_crops(self, session, crops, obj_bbs=None, batch_size=256):
@@ -221,7 +224,7 @@ class Codebook(object):
             batch, bbs = batch_fn(a, e)
             embedding_z[a:e] = session.run(self._encoder.z, feed_dict={self._encoder.x: batch})
             if self.embed_bb and bbs is not None:
-                obj_bbs[a:e] = bbs
+                obj_bbs[a:e] = bbs.cpu().numpy() if isinstance(bbs, torch.Tensor) else bbs
         normalized_embedding = embedding_z / np.linalg.norm(embedding_z, axis=1, keepdims=True)
         session.run(self.embedding_assign_op, {self.embedding: normalized_embedding})
         if self.embed_bb:

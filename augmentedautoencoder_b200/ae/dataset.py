@@ -1,7 +1,8 @@
 """The slice of auto_pose/ae/dataset.py the hot path touches: crop shape, the idx -> rotation table
 (``viewsphere_for_embedding``, dataset.py:39-58, built on pysixd_stuff/view_sampler.py:19-188), ``embedding_size``
 and the square-patch crop helper (dataset.py:354-373).  Rendering / augmentation (OpenGL, imgaug) are out of scope
-(SURVEY.md section 2 rows 7, 11): ``render_embedding_image_batch`` delegates to a user-supplied renderer."""
+(SURVEY.md section 2 rows 7, 11): ``render_embedding_image_batch`` and ``render_training_images`` render with the CUDA
+renderer of augmentedautoencoder_b200/meshrenderer when MODEL_PATH is configured, or call a user-supplied renderer."""
 import math
 
 import numpy as np
@@ -93,6 +94,33 @@ def viewsphere_rotations(min_n_views, num_cyclo, radius):
     return rs
 
 
+def calc_2d_bbox(covered, im_size):
+    """view_sampler.calc_2d_bbox (ae/pysixd_stuff/view_sampler.py:10-15) of the covered pixels: min / max +-1 pixel, clamped to
+    (W - 1, H - 1); [x, y, w, h]"""
+    ys, xs = np.nonzero(covered)
+    x0, y0 = max(xs.min() - 1, 0), max(ys.min() - 1, 0)
+    x1, y1 = min(xs.max() + 1, im_size[0] - 1), min(ys.max() + 1, im_size[1] - 1)
+    return [x0, y0, x1 - x0, y1 - y0]
+
+
+def random_rotation_matrix():
+    """pysixd transform.random_rotation_matrix (ae/pysixd_stuff/transform.py:1463-1503): a uniform random unit quaternion from
+    np.random.rand(3), as a homogeneous 4x4 rotation"""
+    rand = np.random.rand(3)
+    r1, r2 = np.sqrt(1.0 - rand[0]), np.sqrt(rand[0])
+    t1, t2 = math.pi * 2.0 * rand[1], math.pi * 2.0 * rand[2]
+    q = np.array([np.cos(t2) * r2, np.sin(t1) * r1, np.cos(t1) * r1, np.sin(t2) * r2], dtype=np.float64)
+    n = np.dot(q, q)
+    if n < np.finfo(float).eps * 4.0:
+        return np.identity(4)
+    q *= math.sqrt(2.0 / n)
+    q = np.outer(q, q)
+    return np.array([[1.0 - q[2, 2] - q[3, 3], q[1, 2] - q[3, 0], q[1, 3] + q[2, 0], 0.0],
+                     [q[1, 2] + q[3, 0], 1.0 - q[1, 1] - q[3, 3], q[2, 3] - q[1, 0], 0.0],
+                     [q[1, 3] - q[2, 0], q[2, 3] + q[1, 0], 1.0 - q[1, 1] - q[2, 2], 0.0],
+                     [0.0, 0.0, 0.0, 1.0]])
+
+
 class Dataset(object):
     """Constructor signature of auto_pose/ae/dataset.py:16-36 (``Dataset(dataset_path, **kw)`` with the lower-cased
     cfg keys).  Only what the encoder / codebook path needs is kept."""
@@ -115,12 +143,51 @@ class Dataset(object):
     def embedding_size(self):
         return len(self.viewsphere_for_embedding)
 
+    # ------------------------------------------------------------------------------------------------ rendering
+    @property
+    def has_gpu_renderer(self):
+        """True when views are rendered by the CUDA renderer: no renderer callable was passed and a MODEL_PATH is configured"""
+        return self._renderer is None and bool(self._kw.get("model_path"))
+
+    @lazy_property
+    def renderer(self):
+        """meshrenderer_phong.Renderer of MODEL_PATH (dataset.py:61-80), built on first use"""
+        kw = self._kw
+        model = str(kw.get("model", "reconst"))
+        if model == "cad":
+            raise NotImplementedError("MODEL: cad (pyassimp meshes, recalculated normals) is not supported; use MODEL: reconst")
+        if model != "reconst":
+            raise ValueError("MODEL must be reconst or cad, got %r" % model)
+        from ..meshrenderer.meshrenderer_phong import Renderer
+        return Renderer([kw["model_path"]], int(kw.get("antialiasing", 1)), self.dataset_path, float(kw.get("vertex_scale", 1.0)))
+
+    def _render_setup(self):
+        kw = self._kw
+        if self.shape[2] != 3:
+            raise NotImplementedError("C = 1 (grayscale) rendering is not supported")
+        W, H = eval(str(kw.get("render_dims", "(720, 540)")))
+        K = np.array(eval(str(kw.get("k", "[1075.65, 0, 720/2, 0, 1073.90, 540/2, 0, 0, 1]")))).reshape(3, 3)
+        t = np.array([0, 0, float(kw["radius"])])
+        return int(W), int(H), K, t, float(kw.get("clip_near", 10)), float(kw.get("clip_far", 10000)), float(kw.get("pad_factor", 1.2))
+
+    def embedding_crops_device(self, start, end):
+        """uint8 crops [n,H,W,3] and obj_bbs int32 [n,4] of codebook rows start..end as CUDA tensors: the views are rendered with
+        the fixed light and cropped without leaving the device (dataset.py:308-352 without the / 255)."""
+        from ..meshrenderer.meshrenderer_phong import fixed_light
+        W, H, K, t, near, far, pad = self._render_setup()
+        out = self.renderer.render_crops_device(0, W, H, K, self.viewsphere_for_embedding[start:end], t, near, far, fixed_light(), pad,
+                                                self.shape[0], self.shape[1])
+        return out["x"], out["obj_bb"]
+
     def render_embedding_image_batch(self, start, end):
-        """(batch [n,H,W,C] float in [0,1], obj_bbs [n,4]) for codebook rows start..end (dataset.py:308-352).  Needs a
-        renderer callable ``renderer(R) -> (bgr uint8 image, depth)``; OpenGL rendering is out of scope here."""
+        """(batch [n,H,W,C] float in [0,1], obj_bbs [n,4]) for codebook rows start..end (dataset.py:308-352).  Renders on the GPU
+        when MODEL_PATH is configured, else through a renderer callable ``renderer(R) -> (bgr uint8 image, depth)``."""
+        if self._renderer is None and self.has_gpu_renderer:
+            crops, bbs = self.embedding_crops_device(start, end)
+            return crops.cpu().numpy() / 255., bbs.cpu().numpy().astype(np.float64)
         if self._renderer is None:
-            raise NotImplementedError("no renderer attached: pass renderer=callable(R)->(bgr, depth) to Dataset, or "
-                                      "build the codebook with Codebook.update_embedding_from_crops")
+            raise NotImplementedError("no renderer attached: configure model_path, pass renderer=callable(R)->(bgr, depth) to "
+                                      "Dataset, or build the codebook with Codebook.update_embedding_from_crops")
         import cv2
         kw = self._kw
         h, w = self.shape[:2]
@@ -129,11 +196,7 @@ class Dataset(object):
         obj_bbs = np.empty((end - start, 4))
         for i, R in enumerate(self.viewsphere_for_embedding[start:end]):
             bgr, depth = self._renderer(R)
-            ys, xs = np.nonzero(depth > 0)
-            size = (depth.shape[1], depth.shape[0])
-            x0, y0 = max(xs.min() - 1, 0), max(ys.min() - 1, 0)
-            x1, y1 = min(xs.max() + 1, size[0] - 1), min(ys.max() + 1, size[1] - 1)
-            obj_bbs[i] = [x0, y0, x1 - x0, y1 - y0]
+            obj_bbs[i] = calc_2d_bbox(depth > 0, (depth.shape[1], depth.shape[0]))
             crop = self.extract_square_patch(bgr, obj_bbs[i], pad_factor, resize=(w, h), interpolation=cv2.INTER_NEAREST)
             batch[i] = crop / 255.
         return batch, obj_bbs
@@ -156,6 +219,75 @@ class Dataset(object):
             crop[:, :(x - left)] = 0
             crop[:, (x + w - left):] = 0
         return cv2.resize(crop, resize, interpolation=interpolation)
+
+    def training_draws(self, n):
+        """The np.random draws of n training images in the reference's order (dataset.py:243-282): per image the rotation
+        (random_rotation_matrix: rand(3)), the random light of x (random(3), rand, rand), then the two bbox offsets
+        (uniform(-MAX_REL_OFFSET, MAX_REL_OFFSET) each).  Returns (Rs [n,3,3], lights [n,6], offsets [n,2])."""
+        from ..meshrenderer.meshrenderer_phong import random_light
+        m = float(self._kw.get("max_rel_offset", 0.20))
+        Rs, lights, offs = np.empty((n, 3, 3)), np.empty((n, 6)), np.empty((n, 2))
+        for i in range(n):
+            Rs[i] = random_rotation_matrix()[:3, :3]
+            lights[i] = random_light()
+            offs[i, 0] = np.random.uniform(-m, m)
+            offs[i, 1] = np.random.uniform(-m, m)
+        return Rs, lights, offs
+
+    def training_images_from_frames(self, bgr_x, depth_x, bgr_y, depth_y, offsets):
+        """(train_x, mask_x, train_y) composed on the host from full frames, as the reference's loop does after its two render
+        calls (dataset.py:271-303): bbox of depth x, crop of bgr x and depth x at the bbox shifted by offsets * (w, h), mask =
+        depth crop == 0, crop of bgr y at the bbox of depth y.  render_training_images computes the same on the device."""
+        import cv2
+        h, w = self.shape[:2]
+        pad = float(self._kw.get("pad_factor", 1.2))
+        xs, ms, ys = [], [], []
+        for i in range(len(bgr_x)):
+            size = (depth_x[i].shape[1], depth_x[i].shape[0])
+            bb = np.array(calc_2d_bbox(depth_x[i] > 0, size))
+            off = bb + np.array([offsets[i][0] * bb[2], offsets[i][1] * bb[3], 0, 0])
+            xs.append(self.extract_square_patch(bgr_x[i], off, pad, resize=(w, h), interpolation=cv2.INTER_NEAREST).astype(np.uint8))
+            ms.append(self.extract_square_patch(depth_x[i], off, pad, resize=(w, h), interpolation=cv2.INTER_NEAREST) == 0.)
+            bb_y = calc_2d_bbox(depth_y[i] > 0, size)
+            ys.append(self.extract_square_patch(bgr_y[i], bb_y, pad, resize=(w, h), interpolation=cv2.INTER_NEAREST).astype(np.uint8))
+        return np.array(xs), np.array(ms), np.array(ys)
+
+    def render_training_images(self, batch=4096):
+        """train_x (uint8), mask_x (bool) and train_y (uint8) of NOOF_TRAINING_IMGS images (dataset.py:219-306): x with a random
+        light cropped around its bbox shifted by the random offset, its background mask, y with the fixed light around the
+        unshifted bbox.  One render call per batch produces all three without materialising a frame."""
+        from ..meshrenderer.meshrenderer_phong import fixed_light
+        n = int(self._kw["noof_training_imgs"])
+        W, H, K, t, near, far, pad = self._render_setup()
+        h, w = self.shape[:2]
+        Rs, lights, offs = self.training_draws(n)
+        self.train_x = np.empty((n,) + self.shape, np.uint8)
+        self.mask_x = np.empty((n, h, w), bool)
+        self.train_y = np.empty((n,) + self.shape, np.uint8)
+        for a in range(0, n, batch):
+            e = min(n, a + batch)
+            out = self.renderer.render_crops_device(0, W, H, K, Rs[a:e], t, near, far, lights[a:e], pad, h, w, lights_y=fixed_light(),
+                                                    offsets=offs[a:e], want_mask=True, check=False)
+            self.renderer.check_flags(out["flags"].cpu().numpy(), first=a)
+            self.train_x[a:e] = out["x"].cpu().numpy()
+            self.mask_x[a:e] = out["mask"].cpu().numpy()
+            self.train_y[a:e] = out["y"].cpu().numpy()
+        self.noof_training_imgs = n
+
+    def get_training_images(self, dataset_path, args):
+        """Load the cached training set for this cfg or render and cache it (dataset.py:83-97).  The cache file name is the md5
+        of the [Dataset] and [Paths] items, as the reference names it, so caches written by either side load in the other."""
+        import hashlib
+        import os
+        digest = hashlib.md5((str(args.items("Dataset") + args.items("Paths"))).encode("utf-8")).hexdigest()
+        name = os.path.join(dataset_path, digest + ".npz")
+        if os.path.exists(name):
+            self.load_training_images(name)
+        else:
+            self.render_training_images()
+            np.savez(name, train_x=self.train_x, mask_x=self.mask_x, train_y=self.train_y)
+        self.noof_obj_pixels = np.count_nonzero(self.mask_x == 0, axis=(1, 2))
+        return name
 
     # ------------------------------------------------------------------------------------------------ training batches
     def load_training_images(self, path, bg_path=None):

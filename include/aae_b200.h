@@ -71,6 +71,7 @@ typedef struct aae_encoder aae_encoder;
 typedef struct aae_decoder aae_decoder;
 typedef struct aae_codebook aae_codebook;
 typedef struct aae_trainer aae_trainer;
+typedef struct aae_mesh aae_mesh;
 
 AAE_API int aae_version(void);
 AAE_API const char* aae_last_error_string(void);
@@ -229,6 +230,41 @@ AAE_API int aae_trainer_profile(aae_trainer* h, int enable, float* phase_ms_out,
  * boxes (truncated to int like the reference); out_dev: NHWC uint8 [n, out_size, out_size, 3]. */
 AAE_API int aae_extract_square_patches(const uint8_t* image_dev, int img_h, int img_w, const float* boxes_xywh_dev,
                                        int n_boxes, float pad_factor, int out_size, uint8_t* out_dev, void* stream);
+
+/* ---------------------------------------------------------------- Mesh renderer ------------
+ * Batched rasteriser of the reference's phong renderer (auto_pose/meshrenderer/meshrenderer_phong.py, shader
+ * depth_shader_phong.{vs,frag}; MODEL: reconst, ANTIALIASING: 1).  DESIGN.md "Renderer" states the contract and the fp32
+ * operation order.  vertices: host float32 [n_vertices, 9] = position * vertex_scale, normal, colour / 255;
+ * faces: host int32 [n_faces, 3], drawn in this order (equal depth: the earlier triangle wins).
+ * views_dev: float32 [n_views, AAE_RENDER_VIEW_FLOATS] per view: [0:16] view matrix (row-major, the camera's T_view_world),
+ * [16:32] projection (T_proj_view), [32:48] transpose(inverse(view)), [48:54] light 0 = (x, y, z, ambient, diffuse,
+ * specular) in eye coordinates, [54:60] light 1, [60:64] unused.
+ * workspace_dev: at least aae_render_workspace_bytes(mesh, n_views, W, H) bytes of device memory.
+ * flags_dev: int32 [n_views], AAE_RENDER_* bits; a view with AAE_RENDER_BEHIND_CAMERA (a vertex at camera z <= near) is
+ * not rasterised.  obj_bb_dev: int32 [n_views, 4] = calc_2d_bbox of the covered pixels (x, y, w, h). */
+#define AAE_RENDER_VIEW_FLOATS 64
+#define AAE_RENDER_BEHIND_CAMERA 1
+#define AAE_RENDER_EMPTY 2
+#define AAE_RENDER_BAD_CROP 4
+AAE_API int aae_mesh_create(int device, const float* vertices, int64_t n_vertices, const int32_t* faces, int64_t n_faces,
+                            aae_mesh** out);
+AAE_API int aae_mesh_destroy(aae_mesh* h);
+AAE_API int64_t aae_render_workspace_bytes(const aae_mesh* h, int n_views, int W, int H);
+/* Full frames with light 0: bgr_dev uint8 [n, H, W, 3] (BGR, row 0 = top), depth_dev float32 [n, H, W] (camera z, 0 where
+ * nothing was drawn). */
+AAE_API int aae_render_frames(const aae_mesh* h, const float* views_dev, int n_views, int W, int H, float near_plane,
+                              float far_plane, void* workspace_dev, int64_t workspace_bytes, uint8_t* bgr_dev, float* depth_dev,
+                              int32_t* obj_bb_dev, int32_t* flags_dev, void* stream);
+/* Square crops without materialising the frames (Dataset.extract_square_patch + cv2.resize INTER_NEAREST of the frame):
+ * crop_x_dev uint8 [n, out_h, out_w, 3] with light 0 around obj_bb shifted by offsets_dev[v] * (w, h) (float64 [n, 2], NULL:
+ * no shift); mask_x_dev uint8 [n, out_h, out_w] = 1 where crop x shows no object (NULL: not written); crop_y_dev (NULL: not
+ * written) with light 1 around the unshifted obj_bb.  col_map_dev int32 [W + 1, out_w] / row_map_dev int32 [H + 1, out_h]:
+ * row s is the INTER_NEAREST source index of every output column / row for a source of size s. */
+AAE_API int aae_render_crops(const aae_mesh* h, const float* views_dev, int n_views, int W, int H, float near_plane,
+                             float far_plane, const double* offsets_dev, double pad_factor, int out_h, int out_w,
+                             const int32_t* col_map_dev, const int32_t* row_map_dev, void* workspace_dev, int64_t workspace_bytes,
+                             uint8_t* crop_x_dev, uint8_t* mask_x_dev, uint8_t* crop_y_dev, int32_t* obj_bb_dev, int32_t* flags_dev,
+                             void* stream);
 
 #ifdef __cplusplus
 }

@@ -385,13 +385,10 @@ int launch_splitk_reduce(const float* partials, int splits, int64_t MN, int N, c
                          cudaStream_t stream) {
   const int threads = 256;
   // This small kernel sits between kernels that use ~200 KB of shared memory per CTA (the dense GEMM before it, the fused match
-  // after it).  Asking for the same carveout avoids an L1/shared-memory reconfiguration of every SM on both sides
-  // (AAE_NO_CARVEOUT_HINT=1 leaves the default, for A/B measurements).
+  // after it).  Asking for the same carveout avoids an L1/shared-memory reconfiguration of every SM on both sides.
   static const bool hinted = [] {
-    if (getenv("AAE_NO_CARVEOUT_HINT") == nullptr) {
-      cudaFuncSetAttribute(splitk_reduce_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-      cudaFuncSetAttribute(splitk_reduce4_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    }
+    cudaFuncSetAttribute(splitk_reduce_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    cudaFuncSetAttribute(splitk_reduce4_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     return true;
   }();
   (void)hinted;

@@ -26,6 +26,9 @@ constexpr int C1_ATOM = 128 * 128;                 // 128 rows x 128 B
 constexpr int C1_STAGE = 4 * C1_ATOM;              // hi k[0,64), hi k[64,128), lo k[0,64), lo k[64,128)
 constexpr int C1_STAGES = 1;                       // the build (~0.4k cycles) is short next to the MMAs + epilogue; smem goes to the output staging
 constexpr int C1_OUT_LD = 1040;                    // staged output: 32 blocks of 1 KB (one space-to-depth position each), padded against bank conflicts
+// consecutive 1 KB output blocks shipped by one bulk store: fewer, larger copies vs bank conflicts.  Measured 0.25 / 0.22 / 0.28 /
+// 0.28 ms for groups of 1 / 2 / 4 / 8.
+constexpr int C1_OUT_GROUP = 2;
 constexpr int C1_KPAD = 80;
 constexpr int C1_EPI_WARPS = 8;                    // two per TMEM lane quadrant (each takes every other 32-channel chunk)
 constexpr int C1_MMA_WARP = 4 + C1_EPI_WARPS;
@@ -39,7 +42,6 @@ struct Conv1Params {
   int OH, OW, N;           // output dims, N = Cout (<= 128)
   int pad_t, pad_l;
   int num_tiles;
-  int out_group;           // consecutive 1 KB output blocks shipped by one bulk store (1, 2, 4, 8): fewer, larger copies vs bank conflicts
   const float* bias;
   float unscale, out_scale, in_scale;
   __half* out_hi;
@@ -216,7 +218,7 @@ tc_conv1_kernel(const __grid_constant__ CUtensorMap tm_w_hi, const __grid_consta
     const int q = warp & 3, half = (warp - 4) >> 2, r = q * 32 + lane;
     const int ow = r % p.OW, dr = r / p.OW;
     // blocks are grouped G at a time (contiguous, one bulk store per group); 16 bytes of padding after every group
-    const int G = p.out_group, grp_ld = G * 8 * N + 16;
+    constexpr int G = C1_OUT_GROUP, grp_ld = G * 8 * N + 16;
     uint8_t* my_hi = out_smem + ((ow >> 1) / G) * grp_ld + ((ow >> 1) % G) * (8 * N) + (((dr & 1) << 1) | (ow & 1)) * (2 * N);
     uint8_t* my_lo = my_hi + 32 * C1_OUT_LD;
     for (int i = 0; i < my_tiles; ++i) {
@@ -309,7 +311,7 @@ tc_conv1_kernel(const __grid_constant__ CUtensorMap tm_w_hi, const __grid_consta
 
 
 // =====================================================================================================================
-// uint8 feed, second generation (default for uint8 crops; AAE_C1_V1=1 selects the kernel above for same-box A/B runs).
+// uint8 feed, second generation (the path for uint8 crops; the kernel above takes those whose pointer is not 16-byte aligned).
 // The first kernel ran at 0.35 of the HBM write roofline: 3.9 k shared-memory wavefronts per 128-pixel tile against an HBM
 // budget of 2.8 k cycles per tile.  What changed:
 //   * 1/255 is folded into the packed weights, so the A operand is the BYTE ITSELF as fp16 -- exact, no lo plane: two
@@ -331,8 +333,6 @@ constexpr int U8_W_BYTES = 4 * C1_ATOM;
 constexpr int U8_OUT_BYTES = 4 * C1_ATOM;         // hi ch[0,64), hi ch[64,128), lo ch[0,64), lo ch[64,128): 128 slots x 128 B each
 constexpr int U8_SMEM_TOTAL = U8_W_BYTES + U8_A_STAGES * U8_A_STAGE + U8_OUT_BYTES + 2 * U8_PIX_BUF + 1024 /*align*/ + 256 /*barriers*/;
 
-__device__ __forceinline__ void bulk_wait_read_1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
-
 // four bytes -> four fp16 (exact): 0x6400 | b is the fp16 1024 + b, minus 1024
 __device__ __forceinline__ void bytes_to_half4(uint32_t x, uint32_t& lo2, uint32_t& hi2) {
   const __half2 k1024 = __floats2half2_rn(1024.f, 1024.f);
@@ -342,13 +342,13 @@ __device__ __forceinline__ void bytes_to_half4(uint32_t x, uint32_t& lo2, uint32
   hi2 = *reinterpret_cast<const uint32_t*>(&hb);
 }
 
-// Epilogue warps of the uint8 kernel: 16 (four per TMEM lane quadrant, one 32-channel chunk of the tile each) or 8 (two chunks each).
+// Epilogue warps of the uint8 kernel: 16, four per TMEM lane quadrant, one 32-channel chunk of the tile each.
 // In-kernel trace (profiles/r02_conv1_trace.txt): the epilogue paces the kernel -- one chunk costs a warp ~1.7 k cycles of mostly
 // latency (TMEM load, split, proxy fence, tensor-store issue), the builders and the MMAs are far ahead.
-constexpr int U8_MAX_EPI_WARPS = 16;
-constexpr int U8_MAX_THREADS = 32 * (4 + U8_MAX_EPI_WARPS + 1);
+constexpr int U8_EPI_WARPS = 16;
+constexpr int U8_THREADS = 32 * (4 + U8_EPI_WARPS + 1);
 
-__global__ void __launch_bounds__(U8_MAX_THREADS, 1)
+__global__ void __launch_bounds__(U8_THREADS, 1)
 tc_conv1_u8_kernel(const __grid_constant__ CUtensorMap tm_w_hi, const __grid_constant__ CUtensorMap tm_w_lo,
                    const __grid_constant__ CUtensorMap tm_out_hi, const __grid_constant__ CUtensorMap tm_out_lo, const Conv1Params p) {
   constexpr int N = 128, CIN = 3;
@@ -367,7 +367,7 @@ tc_conv1_u8_kernel(const __grid_constant__ CUtensorMap tm_w_hi, const __grid_con
   __shared__ float bias_s[N];
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int n_epi = ((int)blockDim.x >> 5) - 5, mma_warp = 4 + n_epi;      // 8 or 16 epilogue warps, then the issuer warp
+  constexpr int n_epi = U8_EPI_WARPS, mma_warp = 4 + n_epi;                 // the epilogue warps, then the issuer warp
   constexpr int TMEM_COLS = 2 * N;
   if (threadIdx.x < N) bias_s[threadIdx.x] = p.bias[threadIdx.x] * p.out_scale;     // relu(x) * s == relu(x * s) for s > 0
   for (int i = threadIdx.x; i < 2 * U8_PIX_BUF / 4; i += blockDim.x) reinterpret_cast<uint32_t*>(pix)[i] = 0u;   // lead-in / tail stay zero
@@ -458,11 +458,11 @@ tc_conv1_u8_kernel(const __grid_constant__ CUtensorMap tm_w_hi, const __grid_con
   } else if (warp < mma_warp) {
     // ===================== epilogue: TMEM -> bias + ReLU + (hi, lo) split -> swizzled staging -> TMA tensor stores =====================
     // Warp (q, g) owns the tile's slots [32 q, 32 q + 32) and the 32-channel chunks g, g + groups, ... (groups = n_epi / 4: one
-    // chunk per tile with sixteen warps, two with eight).  A chunk goes through 4 KB of the warp's own staging (hi 2 KB, lo 2 KB,
-    // 64-byte rows, 64-byte swizzle: conflict-free STS.128 from a thread-per-slot warp) and is shipped by the warp's own lane 0, so
-    // the tile's tensor stores are issued by n_epi lanes in parallel and no barrier couples the warps.  Sixteen warps: one buffer,
-    // reused a whole tile later; eight warps: one buffer per chunk, the stores of one drain under the math of the other.
-    const int q = warp & 3, g = (warp - 4) >> 2, groups = n_epi >> 2, per_warp = 4 / groups;
+    // chunk per tile).  A chunk goes through 4 KB of the warp's own staging (hi 2 KB, lo 2 KB, 64-byte rows, 64-byte swizzle:
+    // conflict-free STS.128 from a thread-per-slot warp) and is shipped by the warp's own lane 0, so the tile's tensor stores are
+    // issued by n_epi lanes in parallel and no barrier couples the warps.  The buffer is reused a whole tile later.
+    constexpr int groups = n_epi >> 2, per_warp = 4 / groups;
+    const int q = warp & 3, g = (warp - 4) >> 2;
     const float us = p.unscale * p.out_scale;
     const int rsw = (lane >> 1) & 3;
     uint8_t* wbuf = out_smem + (warp - 4) * (U8_OUT_BYTES / n_epi);
@@ -496,7 +496,7 @@ tc_conv1_u8_kernel(const __grid_constant__ CUtensorMap tm_w_hi, const __grid_con
         }
         if (p.range_flag != nullptr && !(amax < 65520.f)) atomicOr(p.range_flag, 1u);
         if (ph >= per_warp) {                            // the buffer was shipped per_warp chunks ago: only newer groups may still be unread
-          if (lane == 0) { if (per_warp == 2) bulk_wait_read_1(); else bulk_wait_read_all(); }
+          if (lane == 0) bulk_wait_read_all();
           __syncwarp();
         }
         uint8_t* sb = wbuf + cc * 4096;
@@ -624,7 +624,7 @@ int tc_conv1_create(int device, const aae_net_cfg* cfg, TcConv1** out) {
   const uint32_t box[2] = {64, (uint32_t)h->N};
   int st = make_tmap_f16(&h->tm_hi, h->w_hi, 2, dims, strides, box);
   if (st == AAE_OK) st = make_tmap_f16(&h->tm_lo, h->w_lo, 2, dims, strides, box);
-  if (st == AAE_OK && h->N == 128 && getenv("AAE_C1_V1") == nullptr) {
+  if (st == AAE_OK && h->N == 128) {
     e = cudaMalloc(&h->w8_hi, (size_t)h->N * 128 * sizeof(__half));
     if (e == cudaSuccess) e = cudaMalloc(&h->w8_lo, (size_t)h->N * 128 * sizeof(__half));
     if (e != cudaSuccess) { set_error("tc conv1 alloc failed: %s", cudaGetErrorString(e)); tc_conv1_destroy(h); return AAE_ERR_OOM; }
@@ -666,10 +666,6 @@ int tc_conv1_forward(TcConv1* h, const aae_net_cfg* cfg, const void* crops, int 
   p.pad_t = std::max((p.OH - 1) * 2 + 5 - p.H, 0) / 2;
   p.pad_l = std::max((p.OW - 1) * 2 + 5 - p.W, 0) / 2;
   p.num_tiles = (int)ceil_div((int64_t)B * p.OH * p.OW, 128);
-  {
-    static const int group = [] { const char* e = getenv("AAE_C1_GROUP"); const int g = e ? atoi(e) : 2; return (g == 1 || g == 2 || g == 4 || g == 8) ? g : 2; }();   // measured: 0.25 / 0.22 / 0.28 / 0.28 ms for 1 / 2 / 4 / 8
-    p.out_group = group;
-  }
   p.bias = bias;
   p.in_scale = act_scale; p.out_scale = act_scale; p.unscale = 1.f / (act_scale * w_scale);
   p.out_hi = out_hi; p.out_lo = out_lo;
@@ -688,8 +684,6 @@ int tc_conv1_forward(TcConv1* h, const aae_net_cfg* cfg, const void* crops, int 
       h->bound_hi = out_hi; h->bound_lo = out_lo; h->slots = slots;
     }
     p.unscale = 1.f / (w_scale * 256.f);              // accumulators hold sum u8 * (w * w_scale * 256 / 255)
-    const char* epi8 = getenv("AAE_C1_EPI8");               // read per launch (scripts/ab_inproc.py): "1" = eight epilogue warps
-    const int u8_threads = 32 * (4 + ((epi8 && epi8[0] == '1') ? 8 : U8_MAX_EPI_WARPS) + 1);
     static long long* trace_dev = nullptr;
     p.trace = nullptr;
     if (getenv("AAE_C1_TRACE")) {
@@ -697,7 +691,7 @@ int tc_conv1_forward(TcConv1* h, const aae_net_cfg* cfg, const void* crops, int 
       cudaMemsetAsync(trace_dev, 0, 96 * sizeof(long long), s);
       p.trace = trace_dev;
     }
-    tc_conv1_u8_kernel<<<grid, u8_threads, U8_SMEM_TOTAL, s>>>(h->tm8_hi, h->tm8_lo, h->tm_out32_hi, h->tm_out32_lo, p);
+    tc_conv1_u8_kernel<<<grid, U8_THREADS, U8_SMEM_TOTAL, s>>>(h->tm8_hi, h->tm8_lo, h->tm_out32_hi, h->tm_out32_lo, p);
     if (p.trace) {
       long long t[96];
       cudaStreamSynchronize(s);

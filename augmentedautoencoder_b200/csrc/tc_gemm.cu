@@ -15,8 +15,8 @@
 // buffer, no stride-2 gathers.  Weights are pre-packed [Cout][25*Cin] K-major.  Both operands land in shared memory in
 // the 128-byte-swizzle canonical layout tcgen05.mma consumes directly.
 //
-// Warp roles (384 threads): warp 0 TMA producer, warp 1 MMA issuer, warp 2 TMEM allocator, warps 4-11 epilogue, two per TMEM lane quadrant
-// (TMEM -> registers -> bias/ReLU -> hi/lo split -> global, in the next layer's space-to-depth layout).
+// Warp roles (512 threads): warp 0 TMA producer, warp 1 MMA issuer, warp 2 TMEM allocator, warps 4-15 epilogue, three per TMEM lane
+// quadrant (TMEM -> registers -> bias/ReLU -> hi/lo split -> global, in the next layer's space-to-depth layout).
 #include <stdlib.h>
 
 #include <algorithm>
@@ -152,15 +152,14 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constan
     }
   } else if (warp >= 4) {
     // ===================== epilogue =====================
-    const int q = warp & 3, half = (warp - 4) >> 2;   // two warps per TMEM lane quadrant, interleaved 32-column chunks
-    const int epi_groups = ((int)blockDim.x >> 5) > 8 ? 2 : 1;
+    const int q = warp & 3, grp = (warp - 4) >> 2;   // TC_EPI_GROUPS warps per TMEM lane quadrant, interleaved 32-column chunks
     const TcRow row = tc_decode_row(p, m0 + q * 32 + lane);
     mbar_wait(tmem_full_bar, 0);
     tc_fence_after();
     const bool has_work = it_end > it_begin;
     const float unscale = p.amax_bits ? p.unscale * tc_dyn_unscale(__ldg(p.amax_bits)) : p.unscale;
 #pragma unroll 1
-    for (int c = half; c < N_TILE / 32; c += epi_groups) {
+    for (int c = grp; c < N_TILE / 32; c += TC_EPI_GROUPS) {
       uint32_t v[32], x[32];
       tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(c * 32), v);
       tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(N_TILE + c * 32), x);
@@ -182,128 +181,21 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constan
 }
 
 
-// ------------------------------------------------------------------------------------------------- 2-CTA kernel
-// Same computation with CTA pairs (cta_group::2): two 128-pixel tiles that share a 256-channel weight tile run as ONE
+// ------------------------------------------------------------------------------------------------- persistent 2-CTA kernel
+// The same computation with CTA pairs (cta_group::2): two 128-pixel tiles that share a 256-channel weight tile run as ONE
 // M = 256 MMA.  Each CTA stages its own pixels plus only HALF of the weight tile (128 channels), so per K chunk it moves
 // 2/3 of the bytes of the single-CTA kernel through L2 -> smem and the tensor core reads 2/3 as much shared memory per
 // MMA -- the single-CTA version is shared-memory-bandwidth bound (operand reads + TMA writes > 128 B/clk/SM).  Both CTAs'
 // TMA loads complete on the leader's (even rank) barrier; the leader's issuer thread fires the MMAs and multicasts the
 // stage-free / accumulator-ready commits to both CTAs; each CTA drains its own 128 TMEM lanes.
-template <int STAGES, int KCH>
 struct TcSmem2 {
+  static constexpr int STAGES = 6;
+  static constexpr int KCH = 32;                          // K chunk per stage (64-byte swizzle)
   static constexpr int T_BYTES = 128 * KCH * 2;          // 128 rows x KCH fp16: A tile and W half tile have the same size
   static constexpr int STAGE_BYTES = 4 * T_BYTES;        // A_hi, A_lo, W_hi(half), W_lo(half)
   static constexpr int TOTAL = STAGES * STAGE_BYTES + 1024 + 256;
 };
 
-template <int STAGES, int KCH>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1)
-tc_gemm2_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ CUtensorMap tm_a_lo,
-                const __grid_constant__ CUtensorMap tm_w_hi, const __grid_constant__ CUtensorMap tm_w_lo, const TcGemmParams p) {
-  using S = TcSmem2<STAGES, KCH>;
-  constexpr int N_TILE = 256;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + STAGES * S::STAGE_BYTES);
-  uint64_t* empty_bar = full_bar + STAGES;
-  uint64_t* tmem_full_bar = empty_bar + STAGES;
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(tmem_full_bar + 1);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const bool leader = rank == 0;
-  const int m0 = blockIdx.x * 128;
-  const int n0 = blockIdx.y * N_TILE;
-  const int total_iters = p.taps * p.chunks_per_tap;
-  const int it_begin = blockIdx.z * p.iters_per_split;          // split-K (OUT_F32 partials): gridDim.z ranges of K iterations
-  const int it_end = min(total_iters, it_begin + p.iters_per_split);
-
-  if (warp == 0 && lane == 0) { prefetch_tmap(&tm_a_hi); prefetch_tmap(&tm_a_lo); prefetch_tmap(&tm_w_hi); prefetch_tmap(&tm_w_lo); }
-  if (warp == 1 && lane == 0) {
-    for (int s = 0; s < STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
-    mbar_init(tmem_full_bar, 1);
-    fence_barrier_init();
-  }
-  if (warp == 2) tmem_alloc_2sm<512>(tmem_ptr);
-  tc_fence_before();
-  cluster_sync_all();   // both CTAs' barriers are initialised before any remote arrival
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      const int hw = p.OH * p.OW;
-      const int b0 = m0 / hw, rem = m0 - b0 * hw;
-      const int oh0 = rem / p.OW, ow0 = rem - oh0 * p.OW;
-      for (int it = it_begin, i = 0; it < it_end; ++it, ++i) {
-        const int s = i % STAGES;
-        mbar_wait(&empty_bar[s], (((uint32_t)(i / STAGES)) & 1u) ^ 1u);
-        const int tap = it / p.chunks_per_tap, cc = it - tap * p.chunks_per_tap;
-        uint8_t* st = smem + s * S::STAGE_BYTES;
-        if (leader) mbar_arrive_expect_tx(&full_bar[s], 2 * S::STAGE_BYTES);   // bytes of both CTAs land on the leader's barrier
-        const uint32_t lb = leader_bar_addr(&full_bar[s]);
-        const int c0 = p.tap_ch[tap] + cc * KCH;
-        const int x = ow0 + p.tap_dj[tap], y = oh0 + p.tap_di[tap];
-        tma_load_4d_2sm(st, &tm_a_hi, lb, c0, x, y, b0);
-        tma_load_4d_2sm(st + S::T_BYTES, &tm_a_lo, lb, c0, x, y, b0);
-        const int kcol = it * KCH;
-        tma_load_2d_2sm(st + 2 * S::T_BYTES, &tm_w_hi, lb, kcol, n0 + (int)rank * 128);
-        tma_load_2d_2sm(st + 3 * S::T_BYTES, &tm_w_lo, lb, kcol, n0 + (int)rank * 128);
-      }
-    }
-  } else if (warp == 1) {
-    if (leader && lane == 0) {
-      constexpr uint32_t idesc = make_idesc_f16(256, N_TILE, 0);
-      for (int it = it_begin, i = 0; it < it_end; ++it, ++i) {
-        const int s = i % STAGES;
-        mbar_wait(&full_bar[s], ((uint32_t)(i / STAGES)) & 1u);
-        tc_fence_after();
-        const uint32_t st = smem_u32(smem + s * S::STAGE_BYTES);
-        const uint64_t a_hi = KCH == 64 ? make_sw128_kmajor_desc(st) : make_sw64_kmajor_desc(st);
-        const uint64_t a_lo = KCH == 64 ? make_sw128_kmajor_desc(st + S::T_BYTES) : make_sw64_kmajor_desc(st + S::T_BYTES);
-        const uint64_t w_hi = KCH == 64 ? make_sw128_kmajor_desc(st + 2 * S::T_BYTES) : make_sw64_kmajor_desc(st + 2 * S::T_BYTES);
-        const uint64_t w_lo = KCH == 64 ? make_sw128_kmajor_desc(st + 3 * S::T_BYTES) : make_sw64_kmajor_desc(st + 3 * S::T_BYTES);
-#pragma unroll
-        for (int k = 0; k < KCH / 16; ++k) {
-          const uint32_t first = (i > 0 || k > 0) ? 1u : 0u;
-          umma_f16_2sm(tmem_base, desc_advance_k(a_hi, k), desc_advance_k(w_hi, k), idesc, first);
-          umma_f16_2sm(tmem_base + N_TILE, desc_advance_k(a_lo, k), desc_advance_k(w_hi, k), idesc, first);
-          umma_f16_2sm(tmem_base + N_TILE, desc_advance_k(a_hi, k), desc_advance_k(w_lo, k), idesc, 1u);
-        }
-        umma_commit_2sm(&empty_bar[s]);
-      }
-      umma_commit_2sm(tmem_full_bar);
-    }
-  } else if (warp >= 4) {
-    const int q = warp & 3, half = (warp - 4) >> 2;   // two warps per TMEM lane quadrant, interleaved 32-column chunks
-    const int epi_groups = ((int)blockDim.x >> 5) > 8 ? 2 : 1;
-    const TcRow row = tc_decode_row(p, m0 + q * 32 + lane);
-    mbar_wait(tmem_full_bar, 0);
-    tc_fence_after();
-    const float unscale = p.amax_bits ? p.unscale * tc_dyn_unscale(__ldg(p.amax_bits)) : p.unscale;
-#pragma unroll 1
-    for (int c = half; c < N_TILE / 32; c += epi_groups) {
-      uint32_t v[32], x[32];
-      tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(c * 32), v);
-      tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(N_TILE + c * 32), x);
-      tmem_ld_wait();
-      const int n = n0 + c * 32;
-      if (!row.valid || n >= p.N) continue;
-      float f[32];
-#pragma unroll
-      for (int j = 0; j < 32; ++j) f[j] = (__uint_as_float(v[j]) + __uint_as_float(x[j])) * unscale;
-      tc_store_chunk(p, row, n, f, (int)blockIdx.z);
-    }
-  }
-  tc_fence_before();
-  cluster_sync_all();   // nobody leaves (or frees TMEM) while the peer may still read this CTA's smem / signal its barriers
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc_2sm<512>(tmem_base);
-  }
-}
-
-// ------------------------------------------------------------------------------------------------- persistent 2-CTA kernel
 // One CTA pair per SM pair walks over the output tiles (m pair fastest, so that concurrently running pairs share the weight
 // tile in L2).  Barrier setup, TMEM allocation and the launch of a fresh CTA are paid once, and the TMA producer runs ahead
 // through the shared-memory ring while the epilogue of the previous tile drains TMEM, so the next tile's MMAs start on full
@@ -316,19 +208,18 @@ __device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
 
 struct TcTileSched {
   int m_pairs, n_tiles, splits;   // tiles = m_pairs * n_tiles * splits, each tile = 256 rows x 256 columns x one K range
-  int late_release;               // A/B: 1 = the epilogue warps release the accumulators only after their last chunk is shipped
   int tma_out;                    // > 0: tm_o_hi / tm_o_lo describe the output and each epilogue warp owns 4 KB of staging behind the ring:
                                   // 1 space-to-depth (hi, lo), 2 plain (hi, lo), 3 depth-to-space (hi, lo), 4 fp32 [M, N] (tm_o_hi only)
   long long* trace;               // AAE_TC_TRACE: clock64 of CTA 0 for its first 96 chunks: [g*4+0] TMA issued, +1 full barrier seen by the MMA thread, +2 MMAs issued, +3 stage seen empty again
 };
 
-template <int STAGES, int KCH>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1)
 tc_gemm2p_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ CUtensorMap tm_a_lo,
                  const __grid_constant__ CUtensorMap tm_w_hi, const __grid_constant__ CUtensorMap tm_w_lo,
                  const __grid_constant__ CUtensorMap tm_o_hi, const __grid_constant__ CUtensorMap tm_o_lo, const TcGemmParams p,
                  const TcTileSched sch) {
-  using S = TcSmem2<STAGES, KCH>;
+  using S = TcSmem2;
+  constexpr int STAGES = S::STAGES, KCH = S::KCH;
   constexpr int N_TILE = 256;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -412,10 +303,10 @@ tc_gemm2p_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_const
           tc_fence_after();
           if (sch.trace && blockIdx.x == 0 && g < 96) sch.trace[g * 4 + 1] = clock64();
           const uint32_t st = smem_u32(smem + s * S::STAGE_BYTES);
-          const uint64_t a_hi = KCH == 64 ? make_sw128_kmajor_desc(st) : make_sw64_kmajor_desc(st);
-          const uint64_t a_lo = KCH == 64 ? make_sw128_kmajor_desc(st + S::T_BYTES) : make_sw64_kmajor_desc(st + S::T_BYTES);
-          const uint64_t w_hi = KCH == 64 ? make_sw128_kmajor_desc(st + 2 * S::T_BYTES) : make_sw64_kmajor_desc(st + 2 * S::T_BYTES);
-          const uint64_t w_lo = KCH == 64 ? make_sw128_kmajor_desc(st + 3 * S::T_BYTES) : make_sw64_kmajor_desc(st + 3 * S::T_BYTES);
+          const uint64_t a_hi = make_sw64_kmajor_desc(st);
+          const uint64_t a_lo = make_sw64_kmajor_desc(st + S::T_BYTES);
+          const uint64_t w_hi = make_sw64_kmajor_desc(st + 2 * S::T_BYTES);
+          const uint64_t w_lo = make_sw64_kmajor_desc(st + 3 * S::T_BYTES);
 #pragma unroll
           for (int k = 0; k < KCH / 16; ++k) {
             const uint32_t first = (i > 0 || k > 0) ? 1u : 0u;
@@ -461,7 +352,7 @@ tc_gemm2p_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_const
           tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(c * 32), v);
           tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(N_TILE + c * 32), x);
           tmem_ld_wait();
-          if (c + epi_groups >= N_TILE / 32 && !sch.late_release) {   // last chunk of this warp: its accumulator words are in registers,
+          if (c + epi_groups >= N_TILE / 32) {                      // last chunk of this warp: its accumulator words are in registers,
             tc_fence_before();                                         // the issuer may overwrite TMEM while the warp finishes the chunk
             __syncwarp();
             if (lane == 0) mbar_arrive_cluster(empty_addr);
@@ -637,82 +528,72 @@ __global__ void __launch_bounds__(256) splitk_forward_finish_kernel(const float*
   }
 }
 
-template <int STAGES, int KCH>
 int launch_tc_gemm2(const TcLayer& L, dim3 grid, cudaStream_t s) {
-  using S = TcSmem2<STAGES, KCH>;
-  auto kern = tc_gemm2_kernel<STAGES, KCH>;
-  AAE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, S::TOTAL));
-  static const bool persistent = getenv("AAE_TC_NOPERSIST") == nullptr;
-  if (persistent) {
-    TcTileSched sch;
-    sch.m_pairs = (int)((grid.x + 1) / 2); sch.n_tiles = (int)grid.y; sch.splits = (int)grid.z;
-    static long long* trace_dev = nullptr;
-    sch.trace = nullptr;
-    if (getenv("AAE_TC_TRACE")) {
-      if (!trace_dev) { cudaMalloc(&trace_dev, (96 * 4 + 8 + 64 + 64) * sizeof(long long)); }
-      cudaMemsetAsync(trace_dev, 0, (96 * 4 + 8 + 64 + 64) * sizeof(long long), s);
-      sch.trace = trace_dev;
-    }
-    const int tiles = sch.m_pairs * sch.n_tiles * sch.splits;
-    auto pk = tc_gemm2p_kernel<STAGES, KCH>;
-    // TMA-store epilogue: 4 KB of staging per epilogue warp behind the ring.  With six 32 KB stages that leaves room for eight
-    // epilogue warps (384 threads); the branch-free epilogue is no longer issue-bound, so eight are enough.
-    const char* no_tma = getenv("AAE_TC_NO_TMA_OUT");            // read per launch (scripts/ab_inproc.py)
-    const bool tma_out_on = !(no_tma && no_tma[0] == '1');
-    constexpr int EPI_TMA = STAGES * S::STAGE_BYTES + 2048 + 12 * 4096 <= 232448 ? 12 : 8;   // epilogue warps the staging has room for
-    const bool f32_target_ok = L.gp.out_mode != OUT_F32 || (sch.splits == 1 && L.gp.out_f32 == L.tma_f32_base);
-    const bool tma_out = tma_out_on && L.tma_out && f32_target_ok && STAGES * S::STAGE_BYTES + 2048 + EPI_TMA * 4096 <= 232448;
-    const int threads = tma_out ? 128 + 32 * EPI_TMA : tc_block_threads();
-    const int smem_bytes = tma_out ? STAGES * S::STAGE_BYTES + 2048 + EPI_TMA * 4096 : S::TOTAL;
-    const char* late = getenv("AAE_TC_LATE_RELEASE");            // read per launch (scripts/ab_inproc.py)
-    sch.late_release = (late && late[0] == '1') ? 1 : 0;
-    sch.tma_out = !tma_out ? 0 : L.gp.out_mode == OUT_S2D_SPLIT ? 1 : L.gp.out_mode == OUT_PLAIN_SPLIT ? 2 : L.gp.out_mode == OUT_D2S_SPLIT ? 3 : 4;
-    AAE_CUDA_OK(cudaFuncSetAttribute(pk, cudaFuncAttributeMaxDynamicSharedMemorySize, std::max(smem_bytes, (int)S::TOTAL)));
-    static int pair_slots = 0;                       // CTA pairs that can be resident at once (asked from the driver: pairs cannot straddle GPCs)
-    if (pair_slots == 0) {
-      int dev = 0, sms = 0;
-      cudaGetDevice(&dev);
-      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-      cudaLaunchConfig_t cfg;
-      memset(&cfg, 0, sizeof(cfg));
-      cfg.gridDim = dim3(2u * (unsigned)std::max(1, sms / 2));
-      cfg.blockDim = dim3((unsigned)threads);
-      cfg.dynamicSmemBytes = (size_t)std::max(smem_bytes, (int)S::TOTAL);
-      cudaLaunchAttribute at;
-      at.id = cudaLaunchAttributeClusterDimension;
-      at.val.clusterDim.x = 2; at.val.clusterDim.y = 1; at.val.clusterDim.z = 1;
-      cfg.attrs = &at; cfg.numAttrs = 1;
-      int n = 0;
-      if (cudaOccupancyMaxActiveClusters(&n, pk, &cfg) != cudaSuccess || n <= 0) { cudaGetLastError(); n = std::max(1, sms / 2); }
-      pair_slots = std::min(n, std::max(1, sms / 2));
-      if (getenv("AAE_TC_VERBOSE")) fprintf(stderr, "[tc] CTA pairs resident at once: %d (of %d SMs / 2 = %d)\n", n, sms, sms / 2);
-    }
-    pk<<<dim3(2u * (unsigned)std::min(tiles, pair_slots)), threads, smem_bytes, s>>>(L.tm_a_hi, L.tm_a_lo, L.tm_w2_hi, L.tm_w2_lo,
-                                                                                   tma_out ? L.tm_o_hi : L.tm_a_hi, tma_out ? L.tm_o_lo : L.tm_a_lo, L.gp, sch);
-    AAE_LAUNCH_OK();
-    if (sch.trace) {
-      long long t[96 * 4 + 8 + 64 + 64];
-      cudaStreamSynchronize(s);
-      cudaMemcpy(t, sch.trace, sizeof(t), cudaMemcpyDeviceToHost);
-      fprintf(stderr, "[gemm2p trace] N=%d taps=%d chunks/tap=%d: chunk: issue | +full seen | +mma issued | next-use empty seen (clocks, relative to chunk 0 issue)\n", L.gp.N, L.gp.taps, L.gp.chunks_per_tap);
-      fprintf(stderr, "  CTA 0 (epilogue warp 4): %lld cycles in %lld ns -> SM clock %.0f MHz during this kernel\n", t[386] - t[384], t[387] - t[385],
-              1e3 * (double)(t[386] - t[384]) / (double)(t[387] - t[385]));
-      for (int k = 0; k < 4; ++k)
-        fprintf(stderr, "  tile 1, warp 4, chunk round %d: tcgen05.ld %lld | math %lld | wait for buffer %lld | STS + proxy fence %lld | TMA issue %lld | (next round starts +%lld)\n", k,
-                t[456 + k * 8 + 1] - t[456 + k * 8], t[456 + k * 8 + 2] - t[456 + k * 8 + 1], t[456 + k * 8 + 3] - t[456 + k * 8 + 2],
-                t[456 + k * 8 + 4] - t[456 + k * 8 + 3], t[456 + k * 8 + 5] - t[456 + k * 8 + 4], k < 3 ? t[456 + (k + 1) * 8] - t[456 + k * 8 + 5] : 0LL);
-      for (int tl = 0; tl < 15; ++tl)
-        fprintf(stderr, "  tile %2d: epilogue warp 4 sees accumulators at %8lld, done +%6lld | issuer waits for drained TMEM from %8lld for %6lld\n", tl,
-                t[392 + tl * 4 + 2] - t[384], t[392 + tl * 4 + 3] - t[392 + tl * 4 + 2], t[392 + tl * 4 + 0] - t[384], t[392 + tl * 4 + 1] - t[392 + tl * 4 + 0]);
-      for (int g = 0; g < 96; g += (g < 8 ? 1 : 16))
-        fprintf(stderr, "  g=%2d issue %7lld | full +%5lld | mma issued +%5lld | empty seen +%5lld\n", g, t[g * 4] - t[0], t[g * 4 + 1] - t[g * 4], t[g * 4 + 2] - t[g * 4],
-                t[g * 4 + 3] - t[g * 4]);
-    }
-    return AAE_OK;
+  using S = TcSmem2;
+  TcTileSched sch;
+  sch.m_pairs = (int)((grid.x + 1) / 2); sch.n_tiles = (int)grid.y; sch.splits = (int)grid.z;
+  static long long* trace_dev = nullptr;
+  sch.trace = nullptr;
+  if (getenv("AAE_TC_TRACE")) {
+    if (!trace_dev) { cudaMalloc(&trace_dev, (96 * 4 + 8 + 64 + 64) * sizeof(long long)); }
+    cudaMemsetAsync(trace_dev, 0, (96 * 4 + 8 + 64 + 64) * sizeof(long long), s);
+    sch.trace = trace_dev;
   }
-  grid.x = (grid.x + 1) & ~1u;   // whole CTA pairs
-  kern<<<grid, tc_block_threads(), S::TOTAL, s>>>(L.tm_a_hi, L.tm_a_lo, L.tm_w2_hi, L.tm_w2_lo, L.gp);
+  const int tiles = sch.m_pairs * sch.n_tiles * sch.splits;
+  auto pk = tc_gemm2p_kernel;
+  // TMA-store epilogue: 4 KB of staging per epilogue warp behind the ring.  With six 32 KB stages that leaves room for eight
+  // epilogue warps (384 threads); the branch-free epilogue is no longer issue-bound, so eight are enough.
+  // AAE_TC_NO_TMA_OUT=1 (read per launch) selects the plain-store epilogue: the reference the TMA-store epilogue is tested against
+  const char* no_tma = getenv("AAE_TC_NO_TMA_OUT");
+  const bool tma_out_on = !(no_tma && no_tma[0] == '1');
+  constexpr int EPI_TMA = 8;                                     // epilogue warps the staging has room for
+  static_assert(S::STAGES * S::STAGE_BYTES + 2048 + EPI_TMA * 4096 <= 232448, "TMA-store staging does not fit behind the ring");
+  const bool f32_target_ok = L.gp.out_mode != OUT_F32 || (sch.splits == 1 && L.gp.out_f32 == L.tma_f32_base);
+  const bool tma_out = tma_out_on && L.tma_out && f32_target_ok;
+  const int threads = tma_out ? 128 + 32 * EPI_TMA : TC_THREADS;
+  const int smem_bytes = tma_out ? S::STAGES * S::STAGE_BYTES + 2048 + EPI_TMA * 4096 : S::TOTAL;
+  sch.tma_out = !tma_out ? 0 : L.gp.out_mode == OUT_S2D_SPLIT ? 1 : L.gp.out_mode == OUT_PLAIN_SPLIT ? 2 : L.gp.out_mode == OUT_D2S_SPLIT ? 3 : 4;
+  AAE_CUDA_OK(cudaFuncSetAttribute(pk, cudaFuncAttributeMaxDynamicSharedMemorySize, std::max(smem_bytes, (int)S::TOTAL)));
+  static int pair_slots = 0;                       // CTA pairs that can be resident at once (asked from the driver: pairs cannot straddle GPCs)
+  if (pair_slots == 0) {
+    int dev = 0, sms = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    cudaLaunchConfig_t cfg;
+    memset(&cfg, 0, sizeof(cfg));
+    cfg.gridDim = dim3(2u * (unsigned)std::max(1, sms / 2));
+    cfg.blockDim = dim3((unsigned)threads);
+    cfg.dynamicSmemBytes = (size_t)std::max(smem_bytes, (int)S::TOTAL);
+    cudaLaunchAttribute at;
+    at.id = cudaLaunchAttributeClusterDimension;
+    at.val.clusterDim.x = 2; at.val.clusterDim.y = 1; at.val.clusterDim.z = 1;
+    cfg.attrs = &at; cfg.numAttrs = 1;
+    int n = 0;
+    if (cudaOccupancyMaxActiveClusters(&n, pk, &cfg) != cudaSuccess || n <= 0) { cudaGetLastError(); n = std::max(1, sms / 2); }
+    pair_slots = std::min(n, std::max(1, sms / 2));
+    if (getenv("AAE_TC_VERBOSE")) fprintf(stderr, "[tc] CTA pairs resident at once: %d (of %d SMs / 2 = %d)\n", n, sms, sms / 2);
+  }
+  pk<<<dim3(2u * (unsigned)std::min(tiles, pair_slots)), threads, smem_bytes, s>>>(L.tm_a_hi, L.tm_a_lo, L.tm_w2_hi, L.tm_w2_lo,
+                                                                                 tma_out ? L.tm_o_hi : L.tm_a_hi, tma_out ? L.tm_o_lo : L.tm_a_lo, L.gp, sch);
   AAE_LAUNCH_OK();
+  if (sch.trace) {
+    long long t[96 * 4 + 8 + 64 + 64];
+    cudaStreamSynchronize(s);
+    cudaMemcpy(t, sch.trace, sizeof(t), cudaMemcpyDeviceToHost);
+    fprintf(stderr, "[gemm2p trace] N=%d taps=%d chunks/tap=%d: chunk: issue | +full seen | +mma issued | next-use empty seen (clocks, relative to chunk 0 issue)\n", L.gp.N, L.gp.taps, L.gp.chunks_per_tap);
+    fprintf(stderr, "  CTA 0 (epilogue warp 4): %lld cycles in %lld ns -> SM clock %.0f MHz during this kernel\n", t[386] - t[384], t[387] - t[385],
+            1e3 * (double)(t[386] - t[384]) / (double)(t[387] - t[385]));
+    for (int k = 0; k < 4; ++k)
+      fprintf(stderr, "  tile 1, warp 4, chunk round %d: tcgen05.ld %lld | math %lld | wait for buffer %lld | STS + proxy fence %lld | TMA issue %lld | (next round starts +%lld)\n", k,
+              t[456 + k * 8 + 1] - t[456 + k * 8], t[456 + k * 8 + 2] - t[456 + k * 8 + 1], t[456 + k * 8 + 3] - t[456 + k * 8 + 2],
+              t[456 + k * 8 + 4] - t[456 + k * 8 + 3], t[456 + k * 8 + 5] - t[456 + k * 8 + 4], k < 3 ? t[456 + (k + 1) * 8] - t[456 + k * 8 + 5] : 0LL);
+    for (int tl = 0; tl < 15; ++tl)
+      fprintf(stderr, "  tile %2d: epilogue warp 4 sees accumulators at %8lld, done +%6lld | issuer waits for drained TMEM from %8lld for %6lld\n", tl,
+              t[392 + tl * 4 + 2] - t[384], t[392 + tl * 4 + 3] - t[392 + tl * 4 + 2], t[392 + tl * 4 + 0] - t[384], t[392 + tl * 4 + 1] - t[392 + tl * 4 + 0]);
+    for (int g = 0; g < 96; g += (g < 8 ? 1 : 16))
+      fprintf(stderr, "  g=%2d issue %7lld | full +%5lld | mma issued +%5lld | empty seen +%5lld\n", g, t[g * 4] - t[0], t[g * 4 + 1] - t[g * 4], t[g * 4 + 2] - t[g * 4],
+              t[g * 4 + 3] - t[g * 4]);
+  }
   return AAE_OK;
 }
 
@@ -721,7 +602,7 @@ int launch_tc_gemm(const TcLayer& L, dim3 grid, cudaStream_t s) {
   using S = TcSmem<N_TILE, STAGES, KCH>;
   auto kern = tc_gemm_kernel<N_TILE, STAGES, KCH>;
   AAE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, S::TOTAL));
-  kern<<<grid, tc_block_threads(), S::TOTAL, s>>>(L.tm_a_hi, L.tm_a_lo, L.tm_w_hi, L.tm_w_lo, L.gp);
+  kern<<<grid, TC_THREADS, S::TOTAL, s>>>(L.tm_a_hi, L.tm_a_lo, L.tm_w_hi, L.tm_w_lo, L.gp);
   AAE_LAUNCH_OK();
   return AAE_OK;
 }
@@ -740,15 +621,9 @@ int tc_dev_alloc(void** p, size_t bytes) {
 }
 
 int tc_launch_layer(const TcLayer& T, dim3 grid, cudaStream_t s) {
-  if (T.pair && T.kch == 32) {
-    const char* s5 = getenv("AAE_TC_S5");                         // five stages leave room for twelve epilogue warps' staging
-    return (s5 && s5[0] == '1') ? launch_tc_gemm2<5, 32>(T, grid, s) : launch_tc_gemm2<6, 32>(T, grid, s);
-  }
-  if (T.pair) return launch_tc_gemm2<3, 64>(T, grid, s);
+  if (T.pair && T.kch == 32) return launch_tc_gemm2(T, grid, s);
   if (T.n_tile == 256 && T.kch == 32) return launch_tc_gemm<256, 4, 32>(T, grid, s);
-  if (T.n_tile == 256) return launch_tc_gemm<256, TC_STAGES, 64>(T, grid, s);
   if (T.n_tile == 128 && T.kch == 64) return launch_tc_gemm<128, 3, 64>(T, grid, s);
-  if (T.n_tile == 128 && T.kch == 32) return launch_tc_gemm<128, 6, 32>(T, grid, s);
   if (T.n_tile == 32 && T.kch == 32) return launch_tc_gemm<32, 6, 32>(T, grid, s);
   set_error("tc_launch_layer: no kernel for n_tile=%d kch=%d", T.n_tile, T.kch);
   return AAE_ERR_UNSUPPORTED;
@@ -835,7 +710,7 @@ int tc_encoder_create(int device, const aae_net_cfg* cfg, TcEncoder** out) {
       if (T.in_c % 64 != 0 || T.out_c % 32 != 0) { set_error("AAE_PREC_TC_SPLIT: dense layer needs flat %% 64 == 0 and latent %% 32 == 0"); st = AAE_ERR_UNSUPPORTED; break; }
     }
     T.n_tile = T.out_c >= 256 ? 256 : 128;
-    T.kch = (T.n_tile == 256 && getenv("AAE_TC_KCH64") == nullptr) ? 32 : 64;
+    T.kch = T.n_tile == 256 ? 32 : 64;
     // batch dimension padded to a whole number of TMA boxes, so a tile never addresses rows outside the tensor map
     const int B_pad = (int)ceil_div(B, T.BB) * T.BB;
     const size_t act_alloc = (size_t)B_pad * T.in_h * T.in_w * T.in_c;
@@ -867,7 +742,7 @@ int tc_encoder_create(int device, const aae_net_cfg* cfg, TcEncoder** out) {
       const uint32_t box[2] = {(uint32_t)T.kch, (uint32_t)std::min(T.n_tile, T.out_c)};
       if ((st = make_tmap_f16(&T.tm_w_hi, T.w_hi, 2, dims, strides, box, 2 * T.kch)) != AAE_OK) break;
       if ((st = make_tmap_f16(&T.tm_w_lo, T.w_lo, 2, dims, strides, box, 2 * T.kch)) != AAE_OK) break;
-      T.pair = !dense && T.n_tile == 256 && T.out_c % 256 == 0 && getenv("AAE_TC_1CTA") == nullptr;
+      T.pair = !dense && T.n_tile == 256 && T.out_c % 256 == 0;
       if (T.pair) {
         const uint32_t box2[2] = {(uint32_t)T.kch, 128};
         const int swz2 = 2 * T.kch;
@@ -1000,8 +875,7 @@ int tc_encoder_forward(TcEncoder* h, const void* crops, int src_u8, int B, const
     // Small batches leave most SM pairs idle (conv4 at 32 crops: 16 tiles of 400 K iterations for 74 pairs): split K so that the
     // persistent grid is covered, fold the fp32 partials and apply the real epilogue in splitk_forward_finish_kernel.
     int splits = 1;
-    static const bool fwd_splitk = getenv("AAE_TC_NO_FWD_SPLITK") == nullptr;     // (A/B switch, read once)
-    if (!dense && T.pair && T.gp.out_mode != OUT_F32 && fwd_splitk) {
+    if (!dense && T.pair && T.gp.out_mode != OUT_F32) {
       const int tiles = (int)((grid.x + 1) / 2) * (int)grid.y, total_iters = T.gp.taps * T.gp.chunks_per_tap;
       if (tiles * 2 <= 74) {
         splits = std::min(74 / tiles, std::max(1, total_iters / 24));
@@ -1164,7 +1038,7 @@ int tc_layer_setup_plain(TcLayer& T, int B, bool pair_ok, bool alloc_input) {
     const uint32_t box[2] = {(uint32_t)T.kch, (uint32_t)T.n_tile};
     if ((st = make_tmap_f16(&T.tm_w_hi, T.w_hi, 2, dims, strides, box, 2 * T.kch)) != AAE_OK) return st;
     if ((st = make_tmap_f16(&T.tm_w_lo, T.w_lo, 2, dims, strides, box, 2 * T.kch)) != AAE_OK) return st;
-    T.pair = pair_ok && T.n_tile == 256 && T.gp.N % 256 == 0 && getenv("AAE_TC_1CTA") == nullptr;
+    T.pair = pair_ok && T.n_tile == 256 && T.gp.N % 256 == 0;
     if (T.pair) {
       const uint32_t box2[2] = {(uint32_t)T.kch, 128};
       if ((st = make_tmap_f16(&T.tm_w2_hi, T.w_hi, 2, dims, strides, box2, 2 * T.kch)) != AAE_OK) return st;
@@ -1210,7 +1084,7 @@ int tc_decoder_create(int device, const aae_net_cfg* cfg, TcDecoder** out) {
       T.BW = hh; T.BH = std::min(hh, 128 / T.BW); T.BB = 128 / (T.BW * T.BH);
       g.OH = g.OW = hh;
       if (l < L) { g.N = 4 * cout; T.n_tile = 256; g.relu = 1; g.out_mode = OUT_D2S_SPLIT; }
-      else if (36 * cout <= 128 && T.in_c % 64 == 0 && getenv("AAE_TC_OUT9") == nullptr) {
+      else if (36 * cout <= 128 && T.in_c % 64 == 0) {
         h->sep_out = true;                          // 1x1 GEMM into P, neighbourhood sum in outlayer_gather_kernel
         T.taps = 1; T.kch = 64; g.N = 128; T.n_tile = 128; g.relu = 0; g.out_mode = OUT_F32; g.cout_real = cout;
         st = dev_alloc((void**)&h->out_p, (size_t)ceil_div((int64_t)B * hh * hh, 128) * 128 * 128 * sizeof(float));

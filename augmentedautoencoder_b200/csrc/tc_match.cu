@@ -47,265 +47,9 @@ __device__ __forceinline__ void unpack_best(unsigned long long k, float& s, int&
   idx = (int)(0xFFFFFFFFu - (uint32_t)(k & 0xFFFFFFFFu));
 }
 
-template <int MQ>
-__global__ void __launch_bounds__(256, 1)
-tc_match_kernel(const __grid_constant__ CUtensorMap tm_e_hi, const __grid_constant__ CUtensorMap tm_e_lo, const float* __restrict__ z,
-                int B, int n_rows, int n_tiles, long long row_offset, unsigned long long* __restrict__ best, unsigned int* __restrict__ counter,
-                float* __restrict__ scores_out, int* __restrict__ idx_out, long long* __restrict__ trace) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* e_smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  uint64_t* e_full = reinterpret_cast<uint64_t*>(e_smem + MT_STAGES * MT_STAGE_BYTES);
-  uint64_t* e_empty = e_full + MT_STAGES;
-  uint64_t* acc_full = e_empty + MT_STAGES;
-  uint64_t* acc_empty = acc_full + 2;
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(acc_empty + 2);
-  __shared__ int s_is_last;
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (trace != nullptr && threadIdx.x == 0) {
-    if (blockIdx.x == 0) trace[12] = clock64();
-    unsigned long long g;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(g));
-    trace[256 + blockIdx.x] = (long long)g;
-  }
-
-  if (warp == 0 && lane == 0) { prefetch_tmap(&tm_e_hi); prefetch_tmap(&tm_e_lo); }
-  if (warp == 1 && lane == 0) {
-    for (int s = 0; s < MT_STAGES; ++s) { mbar_init(&e_full[s], 1); mbar_init(&e_empty[s], 1); }
-    for (int s = 0; s < 2; ++s) { mbar_init(&acc_full[s], 1); mbar_init(&acc_empty[s], 4); }
-    fence_barrier_init();
-  }
-  if (trace != nullptr && blockIdx.x == 0 && threadIdx.x == 64) { trace[13] = clock64(); }
-  if (warp == 2) tmem_alloc<512>(tmem_ptr);
-  if (trace != nullptr && blockIdx.x == 0 && threadIdx.x == 64) { trace[14] = clock64(); }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
-  const bool tr = trace != nullptr && blockIdx.x == 0;
-  if (tr && threadIdx.x == 0) trace[0] = clock64();
-  const int my_tiles = (n_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
-  // kick off the first codebook tiles now: their HBM latency overlaps the query prologue below
-  if (warp == 0 && lane == 0) {
-    for (int i = 0; i < my_tiles && i < 1; ++i) {   // stages 1 and 2 serve as the query staging area until the prologue is done
-      const int row0 = ((int)blockIdx.x + i * (int)gridDim.x) * MT_ROWS;
-      uint8_t* st = e_smem + i * MT_STAGE_BYTES;
-      mbar_arrive_expect_tx(&e_full[i], MT_STAGE_BYTES);
-      tma_load_2d(st, &tm_e_hi, &e_full[i], 0, row0);
-      tma_load_2d(st + MT_E_BYTES, &tm_e_hi, &e_full[i], 64, row0);
-      tma_load_2d(st + 2 * MT_E_BYTES, &tm_e_lo, &e_full[i], 0, row0);
-      tma_load_2d(st + 3 * MT_E_BYTES, &tm_e_lo, &e_full[i], 64, row0);
-    }
-  }
-
-  // ---- prologue, phase A (all warps, coalesced): cp.async every query row into the not-yet-used ring stages 1.. as fp32
-  //      (512 B per row, 16-byte chunks XOR-swizzled by the row, so the row-wise writes here and the thread-per-row reads
-  //      of phase B are both bank-conflict free)
-#pragma unroll 4
-  for (int row = warp; row < MQ * 128; row += 8) {
-    const int mq = row >> 7, r = row & 127;
-    cp_async_16(e_smem + (1 + mq) * MT_STAGE_BYTES + r * 512 + ((lane ^ (r & 31)) << 4), z + (long long)(row < B ? row : 0) * 128 + lane * 4,
-                row < B);
-  }
-  if (tr && threadIdx.x == 0) trace[4] = clock64();
-  cp_async_wait_all();
-  if (tr && threadIdx.x == 0) trace[5] = clock64();
-  __syncthreads();
-  if (tr && threadIdx.x == 0) trace[7] = clock64();
-  // ---- phase B: thread (warp%4, lane) owns row r = 32*(warp%4) + lane of query block mq = warp/4 (warps 4-7 -> block 0,
-  //      warps 0-3 -> block 1): sum of squares, tf.nn.l2_normalize's rsqrt(max(ss, 1e-12)), scale by 64, split into fp16
-  //      (hi, lo) and park the row in TMEM as the MMA's A operand (lane = row, column c = K elements 2c, 2c+1) -- the
-  //      queries never occupy shared memory during the main loop.
-  {
-    const int mq = warp >= 4 ? 0 : 1;
-    if (mq < MQ) {
-      const int q = warp & 3, r = q * 32 + lane;
-      const uint8_t* src = e_smem + (1 + mq) * MT_STAGE_BYTES + r * 512;
-      float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
-#pragma unroll 8
-      for (int c = 0; c < 32; ++c) {
-        const float4 v = *reinterpret_cast<const float4*>(src + ((c ^ (r & 31)) << 4));
-        s0 = fmaf(v.x, v.x, s0); s1 = fmaf(v.y, v.y, s1); s2 = fmaf(v.z, v.z, s2); s3 = fmaf(v.w, v.w, s3);
-      }
-      const float ss = fmaxf((s0 + s1) + (s2 + s3), 1e-12f);
-      float y = rsqrtf(ss);
-      y = y * (1.5f - 0.5f * ss * y * y);              // one Newton step: ~1 ulp
-      const float inv = MT_SCALE * y;
-      const uint32_t lane_base = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(mq * 128);
-#pragma unroll 2
-      for (int g = 0; g < 8; ++g) {                    // 16 K elements -> 8 packed columns of Q_hi and of Q_lo
-        uint32_t hi[8], lo[8];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const float4 v = *reinterpret_cast<const float4*>(src + (((g * 4 + j) ^ (r & 31)) << 4));
-          split_f16x2(v.x * inv, v.y * inv, hi[2 * j], lo[2 * j]);
-          split_f16x2(v.z * inv, v.w * inv, hi[2 * j + 1], lo[2 * j + 1]);
-        }
-        tmem_st_32x8(lane_base + (uint32_t)(g * 8), hi);
-        tmem_st_32x8(lane_base + (uint32_t)(64 + g * 8), lo);
-      }
-      tmem_st_wait();
-    }
-  }
-  if (tr && threadIdx.x == 0) trace[8] = clock64();
-  fence_proxy_async_smem();   // the staging area is about to be overwritten by TMA (async proxy)
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  if (tr && threadIdx.x == 0) trace[1] = clock64();
-
-  if (warp == 0) {
-    if (lane == 0) {
-      for (int i = 1; i < my_tiles; ++i) {
-        const int s = i % MT_STAGES;
-        const uint32_t ph = (uint32_t)(i / MT_STAGES) & 1u;
-        mbar_wait(&e_empty[s], ph ^ 1u);
-        const int row0 = ((int)blockIdx.x + i * (int)gridDim.x) * MT_ROWS;
-        uint8_t* st = e_smem + s * MT_STAGE_BYTES;
-        mbar_arrive_expect_tx(&e_full[s], MT_STAGE_BYTES);
-        tma_load_2d(st, &tm_e_hi, &e_full[s], 0, row0);
-        tma_load_2d(st + MT_E_BYTES, &tm_e_hi, &e_full[s], 64, row0);
-        tma_load_2d(st + 2 * MT_E_BYTES, &tm_e_lo, &e_full[s], 0, row0);
-        tma_load_2d(st + 3 * MT_E_BYTES, &tm_e_lo, &e_full[s], 64, row0);
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      constexpr uint32_t idesc = make_idesc_f16(128, MT_ROWS, 0);
-      for (int i = 0; i < my_tiles; ++i) {
-        const int s = i % MT_STAGES;
-        mbar_wait(&e_full[s], (uint32_t)(i / MT_STAGES) & 1u);
-        if (tr && i < 16) trace[16 + i * 8 + 0] = clock64();
-        const uint32_t est = smem_u32(e_smem + s * MT_STAGE_BYTES);
-#pragma unroll 1
-        for (int mq = 0; mq < MQ; ++mq) {
-          const int u = i * MQ + mq, as = u & 1;        // accumulator stage alternates per (tile, query block)
-          mbar_wait(&acc_empty[as], ((uint32_t)(u >> 1) & 1u) ^ 1u);
-          tc_fence_after();
-          if (tr && i < 16) trace[16 + i * 8 + 1 + mq * 2] = clock64();
-          const uint32_t d = tmem_base + (uint32_t)(MT_TMEM_ACC0 + as * MT_ROWS);
-          const uint32_t q_hi = tmem_base + (uint32_t)(mq * 128), q_lo = q_hi + 64;
-#pragma unroll 1
-          for (int kh = 0; kh < 2; ++kh) {
-            const uint64_t e_hi = make_sw128_kmajor_desc(est + kh * MT_E_BYTES);
-            const uint64_t e_lo = make_sw128_kmajor_desc(est + (2 + kh) * MT_E_BYTES);
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-              const uint32_t kc = (uint32_t)((kh * 4 + k) * 8);   // 16 fp16 K elements = 8 packed columns
-              umma_f16_ts(d, q_lo + kc, desc_advance_k(e_hi, k), idesc, (kh > 0 || k > 0) ? 1u : 0u);
-              umma_f16_ts(d, q_hi + kc, desc_advance_k(e_lo, k), idesc, 1u);
-              umma_f16_ts(d, q_hi + kc, desc_advance_k(e_hi, k), idesc, 1u);
-            }
-          }
-          umma_commit(&acc_full[as]);
-          if (tr && i < 16) trace[16 + i * 8 + 2 + mq * 2] = clock64();
-        }
-        umma_commit(&e_empty[s]);
-      }
-    }
-  } else if (warp >= 4) {
-    const int q = warp & 3;
-    float bs0 = -3.0e38f, bs1 = -3.0e38f;   // running best per query block (kept in named registers: the mq loop is rolled)
-    int bi0 = 0x7FFFFFFF, bi1 = 0x7FFFFFFF;
-    for (int i = 0; i < my_tiles; ++i) {
-      const int row0 = ((int)blockIdx.x + i * (int)gridDim.x) * MT_ROWS;
-      const int nvalid = min(MT_ROWS, n_rows - row0);
-#pragma unroll 1
-      for (int mq = 0; mq < MQ; ++mq) {
-        const int u = i * MQ + mq, as = u & 1;
-        float cbs = mq ? bs1 : bs0;
-        int cbi = mq ? bi1 : bi0;
-        mbar_wait(&acc_full[as], (uint32_t)(u >> 1) & 1u);
-        tc_fence_after();
-        if (tr && warp == 4 && lane == 0 && i < 16) trace[16 + i * 8 + 5 + mq] = clock64();
-#pragma unroll 1
-        for (int c = 0; c < MT_ROWS / 64; ++c) {
-          uint32_t v[32], w[32];
-          const uint32_t col = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(MT_TMEM_ACC0 + as * MT_ROWS + c * 64);
-          tmem_ld_32x32(col, v);
-          tmem_ld_32x32(col + 32, w);
-          tmem_ld_wait();
-          if (nvalid < MT_ROWS) {                       // last tile only: padding rows must never win
-#pragma unroll
-            for (int j = 0; j < 32; ++j) {
-              if (c * 64 + j >= nvalid) v[j] = 0xFF800000u;        // -inf
-              if (c * 64 + 32 + j >= nvalid) w[j] = 0xFF800000u;
-            }
-          }
-          // log-depth max of the 64 scores; the (rare) index search only runs when this chunk beats the running best
-          float m[32];
-#pragma unroll
-          for (int j = 0; j < 32; ++j) m[j] = fmaxf(__uint_as_float(v[j]), __uint_as_float(w[j]));
-#pragma unroll
-          for (int st = 16; st >= 1; st >>= 1)
-#pragma unroll
-            for (int j = 0; j < st; ++j) m[j] = fmaxf(m[j], m[j + st]);
-          const float mx = m[0];
-          if (mx > cbs) {                               // strict >: an equal score later in the table never replaces an earlier row
-            int first = 63;
-#pragma unroll
-            for (int j = 31; j >= 0; --j)
-              if (__uint_as_float(w[j]) == mx) first = 32 + j;
-#pragma unroll
-            for (int j = 31; j >= 0; --j)
-              if (__uint_as_float(v[j]) == mx) first = j;          // lowest column holding the maximum
-            cbs = mx;
-            cbi = row0 + c * 64 + first;
-          }
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&acc_empty[as]);
-        if (mq) { bs1 = cbs; bi1 = cbi; } else { bs0 = cbs; bi0 = cbi; }
-      }
-    }
-#pragma unroll
-    for (int mq = 0; mq < MQ; ++mq) {
-      const int qi = mq * 128 + q * 32 + lane;
-      const float fs = mq ? bs1 : bs0;
-      const int fi = mq ? bi1 : bi0;
-      if (qi < B && fi != 0x7FFFFFFF) atomicMax(best + qi, pack_best(fs * (1.f / (MT_SCALE * MT_SCALE)), fi));
-    }
-  }
-  // ---- teardown + last-CTA finalisation ----
-  if (tr && threadIdx.x == 128) trace[2] = clock64();
-  tc_fence_before();
-  __threadfence();
-  __syncthreads();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc<512>(tmem_base);
-  }
-  if (threadIdx.x == 0) {
-    const unsigned int ticket = atomicAdd(counter, 1u);
-    s_is_last = (ticket == gridDim.x - 1);
-  }
-  __syncthreads();
-  if (s_is_last) {
-    __threadfence();
-    for (int qi = threadIdx.x; qi < B; qi += blockDim.x) {
-      const unsigned long long k = atomicExch(best + qi, 0ull);   // read + re-arm
-      float s;
-      int idx;
-      unpack_best(k, s, idx);
-      scores_out[qi] = s;
-      idx_out[qi] = (int)(idx + row_offset);
-    }
-    if (threadIdx.x == 0) *counter = 0u;
-  }
-  if (tr && threadIdx.x == 0) trace[3] = clock64();
-  if (trace != nullptr && threadIdx.x == 0) {
-    unsigned long long g;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(g));
-    trace[512 + blockIdx.x] = (long long)g;
-  }
-}
-
-
 // ------------------------------------------------------------------------------------------------------------------------
-// Second generation of the fused match (default; AAE_MATCH_V1=1 selects the kernel above for same-box A/B runs).
-// Same arithmetic, same operand layouts, same result.  What changed, each item aimed at the fixed costs that dominated the
-// first kernel (20.5 us at B = 1 against a 7.2 us HBM floor):
+// Second generation of the fused match.  The first kernel (since removed) had the same arithmetic and operand layouts; what
+// changed, each item aimed at the fixed costs that dominated it (20.5 us at B = 1 against a 7.2 us HBM floor):
 //   * the codebook stream starts before anything else: thread 0 initialises the barriers, fences and issues the TMA loads
 //     of the first tiles while the TMEM allocation, the query staging and the normalise/split prologue are still to come
 //     (before: after the allocation and a block-wide barrier, and one tile only);
@@ -688,7 +432,6 @@ struct TcCodebook {
   unsigned long long* lists = nullptr;   // [grid][max_batch][8] packed keys of the per-CTA top-k lists (k > 1)
   unsigned int* counter = nullptr;
   long long* trace = nullptr;   // optional clock64 trace of CTA 0 (AAE_MATCH_TRACE=1), diagnostics only
-  bool v1 = false;              // AAE_MATCH_V1=1: first-generation kernel (k = 1, no upright) for A/B runs
 };
 
 constexpr int MT_KMAX = 8;
@@ -721,7 +464,6 @@ int tc_codebook_create(int device, const float* E_dev, int64_t n_rows, int laten
   h->num_cyclo = std::max(1, num_cyclo);
   h->n_up = ceil_div(n_rows, (int64_t)h->num_cyclo);
   h->n_tiles_up = (int)ceil_div(h->n_up, (int64_t)MT_ROWS);
-  h->v1 = getenv("AAE_MATCH_V1") != nullptr;
   cudaDeviceProp prop;
   cudaGetDeviceProperties(&prop, device);
   h->sm_count = std::min(prop.multiProcessorCount, 148);
@@ -755,9 +497,7 @@ int tc_codebook_create(int device, const float* E_dev, int64_t n_rows, int laten
   }
   if (st != AAE_OK) { tc_codebook_destroy(h); return st; }
   auto attr = [&](const void* fn) { return cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, MT_SMEM_TOTAL); };
-  e = attr((const void*)tc_match_kernel<1>);
-  if (e == cudaSuccess) e = attr((const void*)tc_match_kernel<2>);
-  if (e == cudaSuccess) e = attr((const void*)tc_match2_kernel<1, 1>);
+  e = attr((const void*)tc_match2_kernel<1, 1>);
   if (e == cudaSuccess) e = attr((const void*)tc_match2_kernel<2, 1>);
   if (e == cudaSuccess) e = attr((const void*)tc_match2_kernel<1, MT_KMAX>);
   if (e == cudaSuccess) e = attr((const void*)tc_match2_kernel<2, MT_KMAX>);
@@ -772,20 +512,12 @@ void tc_codebook_destroy(TcCodebook* h) {
   delete h;
 }
 
-static void print_trace(TcCodebook* h, int grid, cudaStream_t s) {
+static void print_trace(TcCodebook* h, cudaStream_t s) {
   long long t[768];
   cudaStreamSynchronize(s);
   cudaMemcpy(t, h->trace, sizeof(t), cudaMemcpyDeviceToHost);
-  if (h->v1) {
-    long long e0 = t[256], e1 = t[256], x0 = t[512], x1 = t[512];
-    for (int i = 0; i < grid; ++i) { e0 = std::min(e0, t[256 + i]); e1 = std::max(e1, t[256 + i]); x0 = std::min(x0, t[512 + i]); x1 = std::max(x1, t[512 + i]); }
-    fprintf(stderr, "[match trace] globaltimer ns: CTA entries span %lld, first exit +%lld, last exit +%lld; CTA0 entry +%lld exit +%lld\n", e1 - e0, x0 - e0, x1 - e0, t[256] - e0, t[512] - e0);
-    fprintf(stderr, "[match trace] entry->t0 %lld (alloc begin %lld end %lld) | ", t[0] - t[12], t[13] - t[12], t[14] - t[12]);
-    fprintf(stderr, "[match trace] start->prologue_done %lld  ->loops_done %lld  ->end %lld | cp issued %lld landed %lld synced %lld tmem written %lld\n", t[1] - t[0], t[2] - t[0], t[3] - t[0], t[4] - t[0], t[5] - t[0], t[7] - t[0], t[8] - t[0]);
-  } else {
-    fprintf(stderr, "[match2 trace, CTA 0, clocks from kernel entry] queries staged + TMEM allocated %lld | prologue done %lld | loops done %lld | end %lld\n",
-            t[4] - t[0], t[1] - t[0], t[2] - t[0], t[3] - t[0]);
-  }
+  fprintf(stderr, "[match2 trace, CTA 0, clocks from kernel entry] queries staged + TMEM allocated %lld | prologue done %lld | loops done %lld | end %lld\n",
+          t[4] - t[0], t[1] - t[0], t[2] - t[0], t[3] - t[0]);
   for (int i = 0; i < 6; ++i)
     fprintf(stderr, "  tile %d: e_full %lld | mq0 acc_empty %lld issued %lld | mq1 acc_empty %lld issued %lld | epi acc_full mq0 %lld mq1 %lld\n", i,
             t[16 + i * 8] - t[0], t[16 + i * 8 + 1] - t[0], t[16 + i * 8 + 2] - t[0], t[16 + i * 8 + 3] - t[0], t[16 + i * 8 + 4] - t[0],
@@ -806,16 +538,12 @@ int tc_codebook_match(TcCodebook* h, const float* z_dev, int B, int64_t row_offs
   const CUtensorMap& th = up ? h->tm_hi_up : h->tm_hi;
   const CUtensorMap& tl = up ? h->tm_lo_up : h->tm_lo;
   const int grid = std::min(h->sm_count, n_tiles);
-  const bool v1 = h->v1 && k == 1 && !up;
   for (int a = 0; a < B; a += 256) {
     const int nb = std::min(256, B - a);
     const float* z = z_dev + (size_t)a * 128;
     float* so = scores_out + (size_t)a * k;
     int32_t* io = idx_out + (size_t)a * k;
-    if (v1) {
-      if (nb > 128) tc_match_kernel<2><<<grid, 256, MT_SMEM_TOTAL, s>>>(th, tl, z, nb, n_rows, n_tiles, (long long)row_offset, h->best, h->counter, so, io, h->trace);
-      else tc_match_kernel<1><<<grid, 256, MT_SMEM_TOTAL, s>>>(th, tl, z, nb, n_rows, n_tiles, (long long)row_offset, h->best, h->counter, so, io, h->trace);
-    } else if (k == 1) {
+    if (k == 1) {
       if (nb > 128) tc_match2_kernel<2, 1><<<grid, 256, MT_SMEM_TOTAL, s>>>(th, tl, z, nb, n_rows, n_tiles, idx_mul, (long long)row_offset, 1, h->best, h->lists, h->counter, so, io, h->trace);
       else tc_match2_kernel<1, 1><<<grid, 256, MT_SMEM_TOTAL, s>>>(th, tl, z, nb, n_rows, n_tiles, idx_mul, (long long)row_offset, 1, h->best, h->lists, h->counter, so, io, h->trace);
     } else {
@@ -824,7 +552,7 @@ int tc_codebook_match(TcCodebook* h, const float* z_dev, int B, int64_t row_offs
     }
     AAE_LAUNCH_OK();
   }
-  if (h->trace) print_trace(h, grid, s);
+  if (h->trace) print_trace(h, s);
   return AAE_OK;
 }
 

@@ -1,8 +1,6 @@
 // Execution-plan structures of the tensor-core path, shared by tc_gemm.cu (inference plans, GEMM kernels) and
 // tc_train.cu (backward plans).  Internal to the library.
 #pragma once
-#include <stdlib.h>
-
 #include <vector>
 
 #include "tc.cuh"
@@ -59,16 +57,10 @@ __device__ __forceinline__ float tc_dyn_unscale(unsigned amax_bits) { return __i
 
 constexpr float ACT_SCALE = 16.f;     // activations (and the [0,1] input) are stored as 16 * x
 constexpr float W_SCALE = 256.f;      // weights are stored as 256 * w
-constexpr int TC_STAGES = 2;
 constexpr int TC_THREADS = 512;       // warp 0 TMA, 1 MMA, 2 TMEM allocator, 3 idle, 4-15 epilogue (three per TMEM lane quadrant)
-// Threads actually launched: 512 by default.  Measured in one process (scripts/ab_inproc.py, +-0.1 %): twelve epilogue warps
-// instead of eight take conv2 / conv3 / conv4 from 1.029 / 0.886 / 0.458 to 1.000 / 0.871 / 0.452 ms (the exposed epilogue shrinks);
-// four warps: 1.170 / 0.941 / 0.468.  AAE_TC_EPI8=1 -> 384 threads, AAE_TC_EPI4=1 -> 256 (read per launch: "1" = on).
-inline int tc_block_threads() {
-  const char* e4 = getenv("AAE_TC_EPI4");
-  const char* e8 = getenv("AAE_TC_EPI8");
-  return (e4 && e4[0] == '1') ? 256 : ((e8 && e8[0] == '1') ? 384 : 512);
-}
+// Twelve epilogue warps instead of eight took conv2 / conv3 / conv4 from 1.029 / 0.886 / 0.458 to 1.000 / 0.871 / 0.452 ms (the
+// exposed epilogue shrinks); four warps: 1.170 / 0.941 / 0.468 (measured on a B200 in one process, +-0.1 %).
+constexpr int TC_EPI_GROUPS = (TC_THREADS / 32 - 4) / 4;   // epilogue warps per TMEM lane quadrant: each takes every third 32-column chunk
 
 struct TcLayer {
   int in_h, in_w, in_c, out_h, out_w, out_c;   // conv geometry (input is the space-to-depth tensor [B, in_h/2, in_w/2, 4*in_c])

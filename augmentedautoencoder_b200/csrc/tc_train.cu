@@ -144,15 +144,14 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_consta
       umma_commit(tmem_full_bar);
     }
   } else if (warp >= 4) {
-    const int q4 = warp & 3, half = (warp - 4) >> 2;
-    const int epi_groups = ((int)blockDim.x >> 5) > 8 ? 2 : 1;
+    const int q4 = warp & 3, grp = (warp - 4) >> 2;   // TC_EPI_GROUPS warps per TMEM lane quadrant, interleaved 32-column chunks
     const TcRow row = tc_decode_row(p.ep, m0 + q4 * 32 + lane);
     mbar_wait(tmem_full_bar, 0);
     tc_fence_after();
     const bool has_work = q_end > q_begin;
     const float unscale = p.ep.amax_bits ? p.ep.unscale * tc_dyn_unscale(__ldg(p.ep.amax_bits)) : p.ep.unscale;
 #pragma unroll 1
-    for (int c = half; c < N_TILE / 32; c += epi_groups) {
+    for (int c = grp; c < N_TILE / 32; c += TC_EPI_GROUPS) {
       uint32_t v[32], x[32];
       tmem_ld_32x32(tmem_base + ((uint32_t)(q4 * 32) << 16) + (uint32_t)(c * 32), v);
       tmem_ld_32x32(tmem_base + ((uint32_t)(q4 * 32) << 16) + (uint32_t)(N_TILE + c * 32), x);
@@ -176,7 +175,7 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_consta
 // ------------------------------------------------------------------------------------------------- wgrad on CTA pairs
 // Same contraction with cta_group::2: two M tiles (consecutive (tap, channel-block) pairs) share one 256-column G tile and
 // run as ONE M = 256 MMA; each CTA stages its own X tile and only HALF of the G tile (128 columns), i.e. 32 KB instead of
-// 48 KB per K chunk, which is what bounds the single-CTA kernel (shared-memory bandwidth, see tc_gemm2_kernel).
+// 48 KB per K chunk, which is what bounds the single-CTA kernel (shared-memory bandwidth, see the pair kernel in tc_gemm.cu).
 template <int STAGES>
 struct WgSmem2 {
   static constexpr int KP = 32;
@@ -270,14 +269,13 @@ tc_wgrad2_kernel(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_const
       umma_commit_2sm(tmem_full_bar);
     }
   } else if (warp >= 4) {
-    const int q4 = warp & 3, half = (warp - 4) >> 2;
-    const int epi_groups = ((int)blockDim.x >> 5) > 8 ? 2 : 1;
+    const int q4 = warp & 3, grp = (warp - 4) >> 2;   // TC_EPI_GROUPS warps per TMEM lane quadrant, interleaved 32-column chunks
     const TcRow row = tc_decode_row(p.ep, m0 + q4 * 32 + lane);
     mbar_wait(tmem_full_bar, 0);
     tc_fence_after();
     const float unscale = p.ep.amax_bits ? p.ep.unscale * tc_dyn_unscale(__ldg(p.ep.amax_bits)) : p.ep.unscale;
 #pragma unroll 1
-    for (int c = half; c < N_TILE / 32; c += epi_groups) {
+    for (int c = grp; c < N_TILE / 32; c += TC_EPI_GROUPS) {
       uint32_t v[32], x[32];
       tmem_ld_32x32(tmem_base + ((uint32_t)(q4 * 32) << 16) + (uint32_t)(c * 32), v);
       tmem_ld_32x32(tmem_base + ((uint32_t)(q4 * 32) << 16) + (uint32_t)(N_TILE + c * 32), x);
@@ -642,7 +640,7 @@ int launch_wgrad(const CUtensorMap& xh, const CUtensorMap& xl, const CUtensorMap
   using S = WgSmem<N_TILE, STAGES>;
   auto kern = tc_wgrad_kernel<N_TILE, STAGES>;
   AAE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, S::TOTAL));
-  kern<<<grid, tc_block_threads(), S::TOTAL, s>>>(xh, xl, gh, gl, p);
+  kern<<<grid, TC_THREADS, S::TOTAL, s>>>(xh, xl, gh, gl, p);
   AAE_LAUNCH_OK();
   return AAE_OK;
 }
@@ -654,7 +652,7 @@ int launch_wgrad2(const CUtensorMap& xh, const CUtensorMap& xl, const CUtensorMa
   auto kern = tc_wgrad2_kernel<STAGES>;
   AAE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, S::TOTAL));
   grid.x = (grid.x + 1) & ~1u;
-  kern<<<grid, tc_block_threads(), S::TOTAL, s>>>(xh, xl, gh, gl, p);
+  kern<<<grid, TC_THREADS, S::TOTAL, s>>>(xh, xl, gh, gl, p);
   AAE_LAUNCH_OK();
   return AAE_OK;
 }
@@ -797,7 +795,7 @@ int tc_train_create(TcEncoder* enc, TcDecoder* dec, int max_batch, TcTrainPlan**
     h->units.push_back(U);
     st = add_unit(h->units.back(), F, 4 * F.in_c);
   }
-  if (st == AAE_OK && Le >= 1 && enc->cfg.in_c == 3 && enc->cfg.kernel_size == 5 && enc->layers[0].in_c == 128 && getenv("AAE_C1_WGRAD_SIMT") == nullptr) {
+  if (st == AAE_OK && Le >= 1 && enc->cfg.in_c == 3 && enc->cfg.kernel_size == 5 && enc->layers[0].in_c == 128) {
     // dW1[75, 128] = sum over pixels of im2col(x)[pixel, :75]^T G1[pixel, :]: the same 1x1 wgrad GEMM as the tap-separable output layer
     const TcLayer& F2 = enc->layers[0];                    // conv2: in_h x in_w x in_c are the dims of conv1's output (stored space-to-depth)
     const size_t n = (size_t)B * F2.in_h * F2.in_w * 128;
@@ -919,8 +917,7 @@ int tc_train_unit_wgrad(TcTrainPlan* h, int u, int B, float* dw_out, cudaStream_
   w.ep.amax_bits = h->amax + u;
   w.ep.out_f32 = h->partials;
   dim3 grid((unsigned)m_tiles, (unsigned)n_tiles, (unsigned)splits);
-  if (U.wg_n_tile == 256 && getenv("AAE_WG_1CTA") == nullptr) AAE_TRY((launch_wgrad2<6>(U.tm_x_hi, U.tm_x_lo, U.tm_g_hi, U.tm_g_lo, w, grid, s)));
-  else if (U.wg_n_tile == 256) AAE_TRY((launch_wgrad<256, 4>(U.tm_x_hi, U.tm_x_lo, U.tm_g_hi, U.tm_g_lo, w, grid, s)));
+  if (U.wg_n_tile == 256) AAE_TRY((launch_wgrad2<6>(U.tm_x_hi, U.tm_x_lo, U.tm_g_hi, U.tm_g_lo, w, grid, s)));
   else AAE_TRY((launch_wgrad<64, 6>(U.tm_x_hi, U.tm_x_lo, U.tm_g_hi, U.tm_g_lo, w, grid, s)));
   if (U.gN == U.n_real) return launch_splitk_reduce(h->partials, splits, mn, w.ep.N, nullptr, ACT_NONE, dw_out, s);
   AAE_REQUIRE((size_t)mn <= h->wm_floats, "tc trainer: merged-gradient scratch too small");

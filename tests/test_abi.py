@@ -83,3 +83,16 @@ def test_product_never_imports_the_oracle():
             if f.endswith((".py", ".cu", ".cuh", ".h")):
                 txt = open(os.path.join(dp, f)).read()
                 assert "oracle" not in txt.replace("# oracle", ""), "%s mentions the oracle" % f
+
+
+def test_library_reads_only_the_documented_environment_variables():
+    # DESIGN §7: one test hook and four diagnostics; none of them selects a kernel variant
+    csrc = os.path.join(ROOT, "augmentedautoencoder_b200", "csrc")
+    names = set()
+    for f in os.listdir(csrc):
+        if f.endswith((".cu", ".cuh")):
+            txt = open(os.path.join(csrc, f)).read()
+            found = re.findall(r'getenv\(\s*"(\w+)"\s*\)', txt)
+            assert len(found) == txt.count("getenv("), "%s reads an environment variable whose name is not a literal" % f
+            names.update(found)
+    assert names == {"AAE_TC_NO_TMA_OUT", "AAE_TC_TRACE", "AAE_C1_TRACE", "AAE_MATCH_TRACE", "AAE_TC_VERBOSE"}
